@@ -67,7 +67,13 @@ def parse_args():
     ap.add_argument("--policy-T", type=int, default=400)
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--device-warmup-s", type=float, default=2.0, help="untimed device warm-up before the W warm-up passes")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the observations, rewards and dones of the last timed pass as float32 DIR/<name>.npy "
+                         "(worlds sampled with numpy default_rng(0) to stay under 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload_config(args, n_gpus):
@@ -538,6 +544,25 @@ def config5_leg(local, rank, world, dev, barrier):
     return out
 
 
+def dump_outputs(out, directory, limit=60 * 10**6):
+    """Write what the last ocb_rollout_random pass handed its caller as float32 .npy files: obs [T, P, n, W, H, C],
+    rewards [T, P, n], dones [T, n] for n worlds drawn without replacement by numpy default_rng(0) (all worlds when
+    they fit in `limit` bytes), in increasing world order."""
+    import numpy as np
+    import torch
+    arrays = {"obs": (out["obs"], 2), "rewards": (out["rewards"], 2), "dones": (out["dones"], 1)}
+    N = out["dones"].shape[1]
+    per_world = sum(4 * t.numel() // N for t, _ in arrays.values())
+    n = min(N, limit // per_world)
+    if n < 1:
+        raise SystemExit("bench.py: one world's outputs (%d bytes) exceed the %d-byte dump limit" % (per_world, limit))
+    idx = np.sort(np.random.default_rng(0).choice(N, size=n, replace=False))
+    idx_t = torch.from_numpy(idx).to(out["dones"].device)
+    os.makedirs(directory, exist_ok=True)
+    for name, (t, axis) in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.index_select(axis, idx_t).float().cpu().numpy())
+
+
 # ----------------------------------------------------------------------------- our arm
 def run_ours(args):
     import torch
@@ -560,18 +585,23 @@ def run_ours(args):
     N, K, W, spl = args.worlds, args.steps, args.warmup, args.env_steps_per_pass
     lp = layouts.load_layout(args.layout, HORIZON)
     P = lp.num_players
-    env = B200Overcooked(args.layout, N, local, horizon=HORIZON, seed=0, world_offset=rank * N)
-    if args.lanes or args.tma >= 0:
-        env.set_tuning(args.lanes, bool(max(args.tma, 0)))
+
+    def make_env():
+        e = B200Overcooked(args.layout, N, local, horizon=HORIZON, seed=0, world_offset=rank * N)
+        if args.lanes or args.tma >= 0:
+            e.set_tuning(args.lanes, bool(max(args.tma, 0)))
+        return e
+
+    env = make_env()
     out = env.alloc_rollout(spl, obs=True, actions=False)
     bytes_ws = layouts.io_bytes_per_world_step(lp)
 
-    def run_passes(n_passes, events=None):
+    def run_passes(n_passes, events=None, on=None):
         for _ in range(n_passes):
             if events is not None:  # every launch gets its own event pair on the launching stream
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record()
-            env.rollout_random(spl, out)
+            (on or env).rollout_random(spl, out)
             if events is not None:
                 e1.record()
                 events.append((e0, e1))
@@ -587,11 +617,14 @@ def run_ours(args):
     t_sampler = time.perf_counter()
     # A freshly leased GPU runs its first seconds of work measurably slower (the same binary measured 30 us in the first
     # process of a box and 24.7 us ten seconds later, profiles/README.md): bring the device to its steady state with
-    # untimed launches of the same kernel before the W warm-up passes of the contract.
+    # untimed launches of the same kernel before the W warm-up passes.  They run on a twin of the env, so that the
+    # timed env always starts from the same state and step count and its outputs do not depend on the host's speed.
+    twin = make_env()
     t_dev = time.perf_counter()
     while time.perf_counter() - t_dev < args.device_warmup_s:
-        run_passes(50)
+        run_passes(50, on=twin)
         torch.cuda.synchronize()
+    twin.close()
     run_passes(max(W, 3))
     barrier()
     t_begin = time.perf_counter()
@@ -602,6 +635,8 @@ def run_ours(args):
     stop.record()
     barrier()
     t_end = time.perf_counter()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     ms = torch.tensor([start.elapsed_time(stop)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
