@@ -69,6 +69,7 @@ PROTOTYPES = {
     "ocb_rollout_policy": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _u64, _vp]),
     "ocb_rollout_policy_fused": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _u64, _vp]),
     "ocb_rollout_crossplay_fused": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _u64, _vp]),
+    "ocb_rollout_population_fused": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _u64, _vp]),
     "ocb_rollout_fused_debug_trace": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _vp, _i, _i]),
     "ocb_rollout_mixed_scratch_bytes": (_sz, [_vp]),
     "ocb_rollout_mixed": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _u64, _u64, _vp, _sz, _vp]),

@@ -674,8 +674,8 @@ extern "C" int ocb_rollout_policy_fused(ocb_env* e, ocb_policy* pol, int T, int 
     if (e->P != 2) return fail(OCB_ERR_UNSUPPORTED, "the policy rollout supports 2 players");
     DeviceGuard guard(e->device);
     RolloutParams p = base_params(e);
-    const int rc = ocb_policy_rollout_fused_launch(pol, policy_index, nullptr, p, e->h_tables.W, e->h_tables.H, T, obs_slab, actions, logp,
-                                                   values, reward, done, deterministic, seed,
+    const int rc = ocb_policy_rollout_fused_launch(pol, policy_index, nullptr, false, p, e->h_tables.W, e->h_tables.H, T, obs_slab, actions,
+                                                   logp, values, reward, done, deterministic, seed,
                                                    reinterpret_cast<const uint64_t*>(e->d_step_counter),
                                                    reinterpret_cast<uint64_t*>(e->d_step_counter), stream);
     if (rc != OCB_OK) return rc;
@@ -697,8 +697,30 @@ extern "C" int ocb_rollout_crossplay_fused(ocb_env* e, ocb_policy* pol, int T, c
     if (e->P != 2) return fail(OCB_ERR_UNSUPPORTED, "the policy rollout supports 2 players");
     DeviceGuard guard(e->device);
     RolloutParams p = base_params(e);
-    const int rc = ocb_policy_rollout_fused_launch(pol, 0, tile_policy, p, e->h_tables.W, e->h_tables.H, T, obs_slab, actions, logp,
-                                                   nullptr, reward, done, deterministic, seed,
+    const int rc = ocb_policy_rollout_fused_launch(pol, 0, tile_policy, false, p, e->h_tables.W, e->h_tables.H, T, obs_slab, actions,
+                                                   logp, nullptr, reward, done, deterministic, seed,
+                                                   reinterpret_cast<const uint64_t*>(e->d_step_counter),
+                                                   reinterpret_cast<uint64_t*>(e->d_step_counter), stream);
+    if (rc != OCB_OK) return rc;
+    if (stream_capturing(stream))
+        e->count_stale = true;
+    else
+        e->step_count += (uint64_t)T;
+    return OCB_OK;
+}
+
+// Self-play of a population in one persistent launch: the worlds [128 s, 128 s + 128) are played by weight set
+// slice_policy[s] on both seats, actor + critic — the buffers of ocb_rollout_policy(tile_policy = slice_policy ++
+// slice_policy, values != NULL), bit for bit.  Also writes obs_slab[0].
+extern "C" int ocb_rollout_population_fused(ocb_env* e, ocb_policy* pol, int T, const int32_t* slice_policy, int8_t* obs_slab,
+                                            int32_t* actions, float* logp, float* values, int32_t* reward, int32_t* done,
+                                            int deterministic, uint64_t seed, void* stream) {
+    if (e == nullptr || pol == nullptr) return fail(OCB_ERR_INVALID_ARG, "NULL handle");
+    if (e->P != 2) return fail(OCB_ERR_UNSUPPORTED, "the policy rollout supports 2 players");
+    DeviceGuard guard(e->device);
+    RolloutParams p = base_params(e);
+    const int rc = ocb_policy_rollout_fused_launch(pol, 0, slice_policy, true, p, e->h_tables.W, e->h_tables.H, T, obs_slab, actions,
+                                                   logp, values, reward, done, deterministic, seed,
                                                    reinterpret_cast<const uint64_t*>(e->d_step_counter),
                                                    reinterpret_cast<uint64_t*>(e->d_step_counter), stream);
     if (rc != OCB_OK) return rc;
@@ -727,8 +749,8 @@ extern "C" int ocb_rollout_fused_debug_trace(ocb_env* e, ocb_policy* pol, int T,
         return fail(OCB_ERR_CUDA, "ocb_rollout_fused_debug_trace: %s", cudaGetErrorString(err));
     }
     RolloutParams p = base_params(e);
-    const int rc = ocb_policy_rollout_fused_launch(pol, policy_index, nullptr, p, e->h_tables.W, e->h_tables.H, T, obs_slab, actions, logp,
-                                                   values, reward, done, 0, seed,
+    const int rc = ocb_policy_rollout_fused_launch(pol, policy_index, nullptr, false, p, e->h_tables.W, e->h_tables.H, T, obs_slab, actions,
+                                                   logp, values, reward, done, 0, seed,
                                                    reinterpret_cast<const uint64_t*>(e->d_step_counter),
                                                    reinterpret_cast<uint64_t*>(e->d_step_counter), nullptr, d_trace, u0, n_steps);
     if (rc == OCB_OK) {

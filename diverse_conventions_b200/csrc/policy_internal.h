@@ -7,13 +7,14 @@
 
 // T-step rollout in ONE persistent launch (rollout_fused.cuh): `envp` carries the env's tables and state arrays.
 // tile_policy == nullptr: self-play of weight set `policy_index` (actor + critic); else cross-play with the per-step path's
-// seat-major tile table (actors only, every output buffer optional).  Returns OCB_ERR_UNSUPPORTED (with the reason in
+// seat-major tile table (actors only, every output buffer optional); with `population`, tile_policy is a table by 128-world
+// slice and each slice is self-play of its weight set (actor + critic).  Returns OCB_ERR_UNSUPPORTED (with the reason in
 // ocb_last_error) when the layout / handle cannot run fused.
-int ocb_policy_rollout_fused_launch(ocb_policy* pol, int policy_index, const int32_t* tile_policy, const ocb::RolloutParams& envp,
-                                    int env_w, int env_h, int T, int8_t* obs_slab, int32_t* actions, float* logp, float* values,
-                                    int32_t* reward, int32_t* done, int deterministic, uint64_t seed, const uint64_t* d_offset,
-                                    uint64_t* d_counter, void* stream, long long* d_trace = nullptr, int trace_u0 = 0,
-                                    int trace_n = 0);
+int ocb_policy_rollout_fused_launch(ocb_policy* pol, int policy_index, const int32_t* tile_policy, bool population,
+                                    const ocb::RolloutParams& envp, int env_w, int env_h, int T, int8_t* obs_slab, int32_t* actions,
+                                    float* logp, float* values, int32_t* reward, int32_t* done, int deterministic, uint64_t seed,
+                                    const uint64_t* d_offset, uint64_t* d_counter, void* stream, long long* d_trace = nullptr,
+                                    int trace_u0 = 0, int trace_n = 0);
 
 // bytes of one observation row the handle was built for (W * H * (5 P + 10)); 1 when shapes outside the tensor-core
 // kernels' range run through policy_generic_kernel

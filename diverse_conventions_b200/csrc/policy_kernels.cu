@@ -134,7 +134,9 @@ struct PolicyParams {
     int single;               // policy_pair_kernel: 0 = both networks of a tile, 1 = the actor only, 2 = the critic only (one stream)
     // fused rollout (rollout_fused.cuh): a CTA's virtual tiles come in rounds of f_vt_round = slots * (T + 1); with
     // tile_policy set (cross-play) the round's world tiles 2 c, 2 c + 1 play seat 0 / seat 1 with the actors of
-    // tile_policy[kt / 2] / tile_policy[f_seat1_tiles + kt / 2] (the per-step path's seat-major 128-row tile table)
+    // tile_policy[kt / 2] / tile_policy[f_seat1_tiles + kt / 2] (the per-step path's seat-major 128-row tile table).
+    // Population self-play (the kernel instances with kPop) sets f_seat1_tiles = 0 and a table by 128-world slice: fused_pair
+    // gives p | p << 16 and the two networks are the actor and the critic of weight set p
     int f_vt_round, f_slots, f_seat1_tiles;
 };
 
@@ -903,7 +905,8 @@ __host__ __device__ inline PairSmemLayout pair_smem_layout(int npos, int ring, i
     return s;
 }
 
-template <bool kProf>
+// kPop (population self-play in the fused rollout): the two streams are the actor and critic of the slice's weight set
+template <bool kProf, bool kPop = false>
 __device__ __forceinline__ void pair_producer_role(long long* pw, const PolicyParams& prm, int t0, int t1, const BlobLayout L,
                                                    uint32_t s_head, uint32_t s_wring, uint32_t bars) {
     const int nets = prm.single ? 1 : 2;  // single mode: the one network takes the actor's places (stream 0, ring slots 0, 1, ...)
@@ -920,7 +923,7 @@ __device__ __forceinline__ void pair_producer_role(long long* pw, const PolicyPa
         const int tp = tile_pol(prm, t);
         const bool cross = prm.f_vt_round != 0 && prm.tile_policy != nullptr;  // both streams are actors (of two policies)
         const uint8_t* blob_a = prm.blobs + ((size_t)(cross ? (tp & 0xFFFF) : tp) * 2 + (prm.single == 2 ? 1 : 0)) * prm.blob_stride;
-        const uint8_t* blob_c = cross ? prm.blobs + (size_t)(tp >> 16) * 2 * prm.blob_stride : blob_a + prm.blob_stride;
+        const uint8_t* blob_c = cross && !kPop ? prm.blobs + (size_t)(tp >> 16) * 2 * prm.blob_stride : blob_a + prm.blob_stride;
         if (chg) {
             if (u > 0) mbar_wait_p<kProf>(bars + 8 * (PB_HEAD_EMPTY + ((u - 1) & 1)), ((u - 1) >> 1) & 1, pw[PW_HEAD_EMPTY]);
             if (elect_one()) {
@@ -1130,7 +1133,7 @@ __device__ __forceinline__ void pair_fc_role(long long* pw, const PolicyParams& 
 }
 
 // `out(t, trow_id, g, head)` consumes the head outputs of row trow_id of tile t (g = 0: six logits, g = 1: head[0] = value)
-template <bool kProf, bool kSplit, class Out>
+template <bool kProf, bool kSplit, bool kPop = false, class Out>
 __device__ __forceinline__ void pair_epilogue_role(long long* pw, const PolicyParams& prm, int t0, int t1, const BlobLayout L, uint32_t tmem,
                                                    const uint8_t* s_head, uint32_t bars, Out&& out) {
     const int warp = threadIdx.x >> 5, g = warp >> 2, trow_id = (warp & 3) * 32 + (threadIdx.x & 31);
@@ -1144,7 +1147,7 @@ __device__ __forceinline__ void pair_epilogue_role(long long* pw, const PolicyPa
     const float* s_bh = reinterpret_cast<const float*>(rest + L.bh);
     const uint32_t a2 = trow + kPColA2 + g * kA2Cols;
     // head layout / outputs: 0 = actor (6 logits), 1 = critic (value); fused cross-play: two actors
-    const int net = (prm.f_vt_round != 0 && prm.tile_policy != nullptr) ? 0 : (prm.single == 2 ? 1 : g);
+    const int net = (!kPop && prm.f_vt_round != 0 && prm.tile_policy != nullptr) ? 0 : (prm.single == 2 ? 1 : g);
 
     uint32_t u = 0, head_gen = 0, item = 0, d1_par = 0;  // d1_par: phase parity bit per conv accumulator stage
     int trace_vt = 0, trace_item = 0;
@@ -1664,6 +1667,9 @@ extern "C" int ocb_policy_create(const ocb_config* cfg, int device, int hidden, 
     if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<true, true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<true, false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, false, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, true, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, false, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(conv512_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(gemm512_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(gemm512_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
@@ -2056,21 +2062,27 @@ extern "C" int ocb_policy_debug_profile(ocb_policy* p, const int8_t* obs, int M,
 // tile_policy == nullptr: self-play of weight set `policy_index` with its critic (obs_slab, actions and values required).
 // tile_policy != nullptr: cross-play, the per-step path's seat-major table (int32 [2 N / 128], device); actors only, every
 // output buffer optional.
-int ocb_policy_rollout_fused_launch(ocb_policy* p, int policy_index, const int32_t* tile_policy, const RolloutParams& envp, int env_w,
-                                    int env_h, int T, int8_t* obs_slab, int32_t* actions, float* logp, float* values, int32_t* reward,
-                                    int32_t* done, int deterministic, uint64_t seed, const uint64_t* d_offset,
-                                    uint64_t* d_counter, void* stream, long long* d_trace, int trace_u0, int trace_n) {
+// population: tile_policy is a table by 128-world slice (int32 [N / 128], device); slice s is self-play of weight set
+// tile_policy[s] with its critic (obs_slab, actions and values required).
+int ocb_policy_rollout_fused_launch(ocb_policy* p, int policy_index, const int32_t* tile_policy, bool population,
+                                    const RolloutParams& envp, int env_w, int env_h, int T, int8_t* obs_slab, int32_t* actions,
+                                    float* logp, float* values, int32_t* reward, int32_t* done, int deterministic, uint64_t seed,
+                                    const uint64_t* d_offset, uint64_t* d_counter, void* stream, long long* d_trace, int trace_u0,
+                                    int trace_n) {
     if (p == nullptr) return fail(OCB_ERR_INVALID_ARG, "policy is NULL");
     if (p->generic) return fail(OCB_ERR_UNSUPPORTED, "the fused rollout kernel needs the tensor-core policy path (2 players, grids up to %d rows)", kMaxH);
     if (p->hidden != kHid) return fail(OCB_ERR_UNSUPPORTED, "the fused rollout kernel exists for hidden_size 64 only");
-    const bool cross = tile_policy != nullptr;
-    if (!cross && (policy_index < 0 || policy_index >= p->n_policies)) return fail(OCB_ERR_INVALID_ARG, "policy index out of range");
+    if (population && tile_policy == nullptr) return fail(OCB_ERR_INVALID_ARG, "slice_policy is NULL");
+    const bool cross = tile_policy != nullptr && !population;
+    if (tile_policy == nullptr && (policy_index < 0 || policy_index >= p->n_policies)) return fail(OCB_ERR_INVALID_ARG, "policy index out of range");
     if (env_w != p->W || env_h != p->H) return fail(OCB_ERR_INVALID_ARG, "env and policy were built for different layouts");
     if (T < 1) return fail(OCB_ERR_INVALID_ARG, "T must be >= 1");
     if (!cross && (obs_slab == nullptr || actions == nullptr || values == nullptr))
         return fail(OCB_ERR_INVALID_ARG, "obs_slab, actions and values are required");
     if (cross && (envp.N % kRows) != 0)
         return fail(OCB_ERR_INVALID_ARG, "cross-play needs a multiple of %d worlds (one weight set per 128-row tile of a seat), got %d", kRows, envp.N);
+    if (population && (envp.N % kRows) != 0)
+        return fail(OCB_ERR_INVALID_ARG, "population self-play needs a multiple of %d worlds (one weight set per slice), got %d", kRows, envp.N);
     if (cross && values != nullptr) return fail(OCB_ERR_INVALID_ARG, "the cross-play rollout runs no critic: values must be NULL");
     const int wtiles = (envp.N + kFWorlds - 1) / kFWorlds;
     // two tiles in flight when there are more tiles than SMs and the second tile's planes leave a usable weight ring
@@ -2091,7 +2103,7 @@ int ocb_policy_rollout_fused_launch(ocb_policy* p, int policy_index, const int32
     DeviceGuard guard(p->device);
     FusedParams fp;
     memset(&fp, 0, sizeof(fp));
-    fp.pol.blobs = cross ? p->d_blobs : p->d_blobs + (size_t)policy_index * 2 * (size_t)p->L.total;
+    fp.pol.blobs = tile_policy != nullptr ? p->d_blobs : p->d_blobs + (size_t)policy_index * 2 * (size_t)p->L.total;
     fp.pol.blob_stride = (size_t)p->L.total;
     fp.pol.W = p->W, fp.pol.H = p->H, fp.pol.S = p->S, fp.pol.SC = p->SC, fp.pol.npos = p->npos;
     fp.pol.M = kRows, fp.pol.tiles = 1;
@@ -2099,7 +2111,9 @@ int ocb_policy_rollout_fused_launch(ocb_policy* p, int policy_index, const int32
     fp.pol.rng_rows_per_seat = p->rng_rows_per_seat, fp.pol.rng_add0 = p->rng_add0, fp.pol.rng_add1 = p->rng_add1;
     fp.pol.d_offset = reinterpret_cast<const unsigned long long*>(d_offset);
     fp.pol.net_mask = 3, fp.pol.pair_ring = ring, fp.pol.stage_stride = p->stage_stride;
-    fp.pol.tile_policy = tile_policy, fp.pol.f_vt_round = slots * (T + 1), fp.pol.f_slots = slots, fp.pol.f_seat1_tiles = envp.N / kRows;
+    // a round's world tiles (2 c, 2 c + 1 with two in flight) lie in one 128-world slice, so weights change only between rounds
+    fp.pol.tile_policy = tile_policy, fp.pol.f_vt_round = slots * (T + 1), fp.pol.f_slots = slots;
+    fp.pol.f_seat1_tiles = population ? 0 : envp.N / kRows;
     fp.env = envp;
     fp.T = T, fp.wtiles = wtiles, fp.slots = slots, fp.cross = cross ? 1 : 0;
     fp.obs_slab = obs_slab, fp.actions = actions, fp.logp = logp, fp.values = values, fp.reward = reward, fp.done = done;
@@ -2112,7 +2126,8 @@ int ocb_policy_rollout_fused_launch(ocb_policy* p, int policy_index, const int32
         fp.vec_loader = e != nullptr ? (e[0] != '0') : (p->SC % 16 == 0);
     }
     {   // split mode (the critic's conv stream deferred behind the actor's): needs every grid column of a tile resident, one
-        // tile in flight and a critic
+        // tile in flight and a critic.  Population self-play takes it too: a change of weights between rounds waits, like
+        // every head reload, for the previous tile's head-empty barrier, which counts the deferred critic conv's commit
         const int cols = 192 / (kCellCols * p->H);
         const char* e = getenv("OCB_FUSED_SPLIT");
         const bool want = e != nullptr ? (e[0] != '0') : true;
@@ -2120,7 +2135,17 @@ int ocb_policy_rollout_fused_launch(ocb_policy* p, int policy_index, const int32
         if (fp.col_ring < p->W) fp.col_ring = 0;
     }
     const cudaStream_t st = (cudaStream_t)stream;
-    if (fp.col_ring > 0) {
+    if (population) {  // its own instances: the self-play and cross-play launches keep the code they had without this mode
+        if (fp.col_ring > 0) {
+            rollout_fused_kernel<false, true, 1, true><<<ctas, kFThreads, smem, st>>>(fp);
+        } else {
+            fp.col_ring = kColRing;
+            if (slots == 2)
+                rollout_fused_kernel<false, false, 2, true><<<ctas, kFThreads, smem, st>>>(fp);
+            else
+                rollout_fused_kernel<false, false, 1, true><<<ctas, kFThreads, smem, st>>>(fp);
+        }
+    } else if (fp.col_ring > 0) {
         if (d_trace != nullptr)
             rollout_fused_kernel<true, true, 1><<<ctas, kFThreads, smem, st>>>(fp);
         else

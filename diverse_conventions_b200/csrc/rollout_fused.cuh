@@ -1,7 +1,8 @@
 // rollout_fused.cuh — a whole T-step self-play or cross-play rollout in ONE persistent launch (included by
 // policy_kernels.cu inside its anonymous namespace, after the pair kernel whose roles it reuses).
 // Variants (FusedParams): one or two world tiles in flight per CTA (`slots`), split mode (the critic's conv stream deferred
-// behind the actor's; one tile in flight, whole grid resident in TMEM), cross-play (`cross`: two actors, seat-selected rows).
+// behind the actor's; one tile in flight, whole grid resident in TMEM), cross-play (`cross`: two actors, seat-selected rows),
+// population self-play (`kPop`: the actor + critic of a weight set chosen per 128-world slice).
 //
 // The 2T+1-launch rollout (ocb_rollout_policy) is bound by its dependent launches: per env step a
 // policy launch and an env launch, each of which fills and drains the GPU for one tile per SM.
@@ -44,6 +45,8 @@ struct FusedParams {
     // Cross-play (pol.tile_policy set, xd_player.py:190-207 / partner_agents.py:97-111): seat-0 rows act with the actor of
     // policy tile_policy[seat-0 tile], seat-1 rows with the actor of tile_policy[seat-1 tile]; both actors run over all 128
     // rows of the tile as the pipeline's "two networks" and each epilogue group emits the rows of its seat.  No critic.
+    // Population self-play (kernel instances with kPop, pol.f_seat1_tiles = 0) is not `cross`: the two networks are the
+    // actor and critic of the slice's weight set and every row is emitted, as in self-play.
     int cross;
 };
 
@@ -420,7 +423,7 @@ struct FusedOut {
     }
 };
 
-template <bool kProf, bool kSplit, int kSlots>
+template <bool kProf, bool kSplit, int kSlots, bool kPop = false>
 __global__ void __launch_bounds__(kFThreads, 1) rollout_fused_kernel(const FusedParams fp) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((128u - (smem_addr(smem_raw) & 127u)) & 127u);
@@ -478,7 +481,7 @@ __global__ void __launch_bounds__(kFThreads, 1) rollout_fused_kernel(const Fused
 
     long long pw[kProf ? PW_COUNT : 1] = {};
     if (warp < kEpiWarps) {
-        pair_epilogue_role<kProf, kSplit>(pw, prm, 0, nvt, L, tmem, s_head, bars, FusedOut(fp, s_act, bars));
+        pair_epilogue_role<kProf, kSplit, kPop>(pw, prm, 0, nvt, L, tmem, s_head, bars, FusedOut(fp, s_act, bars));
     } else if (warp < kWarpMma) {
         fused_loader_role<kProf, kSplit>(fp, (uint32_t)nvt, tmem, s_env, sl, bars);
     } else if (warp == kWarpMma || warp == kWarpConv2) {
@@ -489,7 +492,7 @@ __global__ void __launch_bounds__(kFThreads, 1) rollout_fused_kernel(const Fused
         else
             pair_conv_role<kProf, -1>(pw, prm, 0, nvt, L, tmem, smem_addr(s_head), bars, half, 2);
     } else if (warp == kPWarpProd) {
-        pair_producer_role<kProf>(pw, prm, 0, nvt, L, smem_addr(s_head), smem_addr(s_wring), bars);
+        pair_producer_role<kProf, kPop>(pw, prm, 0, nvt, L, smem_addr(s_head), smem_addr(s_wring), bars);
     } else if (warp < kPWarpProd) {
         pair_fc_role<kProf, kSplit>(pw, prm, warp - kWarpFc, 0, nvt, L, tmem, smem_addr(s_wring), bars);
     } else if (warp == kFWarpConvC) {

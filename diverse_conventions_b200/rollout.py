@@ -138,7 +138,11 @@ class PolicyRollout:
 
         ``fused``: run the rollout as ONE persistent launch (``ocb_rollout_policy_fused``: self-play of weight
         set ``policy_index``, hidden 64, critic on); ``None`` = use it whenever it applies, ``False`` = always the
-        2T+1-launch path.  Both paths fill bit-identical buffers."""
+        2T+1-launch path.  Both paths fill bit-identical buffers.  A ``tile_policy`` whose two seat halves are equal
+        (``pair_tile_policy([(p0, p0), (p1, p1), ...], worlds_per_slice)``) with the critic on is population self-play:
+        it runs as one launch too (``ocb_rollout_population_fused``).  The table is classified once, here: the launches
+        read the caller's tensor, so in-place edits take effect (also in graph replays) but must keep the two halves
+        equal; build a new ``PolicyRollout`` for a table that mixes policies across seats."""
         if env.num_players != policy.layout.num_players:
             raise ValueError("env and policy were built for different player counts")
         if env.sim_device != policy.device:
@@ -157,11 +161,23 @@ class PolicyRollout:
         self.policy_index = policy_index
         # one persistent launch needs the tensor-core policy path: 2 players, grids up to 6 rows (else per-step launches,
         # which run any shape — the generic policy kernel covers schelling / corridor / multiplayer_schelling ...)
-        # (self-play of one policy with its critic, or cross-play slices without a critic: ocb_rollout_crossplay_fused)
+        # (self-play of one policy with its critic, or cross-play slices without a critic: ocb_rollout_crossplay_fused,
+        # or self-play slices of a population with their critics: ocb_rollout_population_fused)
         small = policy.hidden == 64 and env.num_players == 2
-        can_fuse = small and ((tile_policy is None and with_critic) or
+        self._slice_policy = None
+        if tile_policy is not None and with_critic and env.num_players == 2 and env.num_envs % TILE == 0:
+            half = tile_policy.numel() // 2
+            host = tile_policy.cpu()
+            if torch.equal(host[:half], host[half:]):
+                self._slice_policy = tile_policy[:half]
+        population = self._slice_policy is not None
+        can_fuse = small and ((tile_policy is None and with_critic) or population or
                               (tile_policy is not None and not with_critic and env.num_envs % TILE == 0))
-        if fused and not can_fuse:
+        if fused and population and not small:
+            raise _native.NativeError(_native.OCB_ERR_UNSUPPORTED, "the population launch exists for hidden_size 64 only")
+        # fused=True on a population table of a layout the fused kernel does not take (generic-kernel layouts, layouts too
+        # large for its shared memory) is answered by the launch itself: OCB_ERR_UNSUPPORTED, raised at collect()
+        if fused and not (can_fuse or population):
             raise ValueError("the fused rollout needs hidden 64, two players and either self-play of one policy with its critic "
                              "or cross-play slices (tile_policy, a multiple of %d worlds) without one" % TILE)
         self.fused = can_fuse if fused is None else bool(fused)
@@ -185,7 +201,12 @@ class PolicyRollout:
         # handle-level state, set per issue: several rollouts may share one policy handle
         _native.check(self._lib.ocb_policy_set_sampling_rows(self.policy._h, *self._sampling_rows))
         if self.fused:
-            if self.tile_policy is not None:
+            if self._slice_policy is not None:
+                rc = self._lib.ocb_rollout_population_fused(
+                    env._h, self.policy._h, self.T, _ptr(self._slice_policy), _ptr(b.obs), _ptr(b.actions),
+                    _ptr(b.action_log_probs), _ptr(b.value_preds), _ptr(b.rewards), _ptr(b.dones), int(deterministic),
+                    self.seed, stream)
+            elif self.tile_policy is not None:
                 rc = self._lib.ocb_rollout_crossplay_fused(
                     env._h, self.policy._h, self.T, _ptr(self.tile_policy), _ptr(b.obs), _ptr(b.actions),
                     _ptr(b.action_log_probs), _ptr(b.rewards), _ptr(b.dones), int(deterministic), self.seed, stream)
@@ -246,6 +267,16 @@ class PolicyRollout:
         rs, ep = self.env.episode_stats()
         n = int(ep.sum().item())
         return float(rs.sum().item()) / n if n else float("nan")
+
+    def slice_episode_returns(self, worlds_per_slice: int):
+        """(sum of episode returns int64 [S], episodes int64 [S]) per contiguous slice of ``worlds_per_slice`` worlds, on
+        the device: the per-member scores of a population trained on self-play slices (as ``CrossPlayEvaluator.run``)"""
+        N = self.env.num_envs
+        if worlds_per_slice <= 0 or N % worlds_per_slice != 0:
+            raise ValueError("worlds_per_slice must divide the env's %d worlds" % N)
+        rs, ep = self.env.episode_stats()
+        n = N // worlds_per_slice
+        return rs.view(n, worlds_per_slice).sum(1), ep.view(n, worlds_per_slice).sum(1, dtype=torch.int64)
 
 
 # ---------------------------------------------------------------------------- cross-play

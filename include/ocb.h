@@ -287,6 +287,19 @@ int ocb_rollout_crossplay_fused(ocb_env* env, ocb_policy* pol, int T, const int3
                                 int32_t* actions, float* logp, int32_t* reward, int32_t* done, int deterministic,
                                 uint64_t seed, void* stream);
 
+/* Self-play of a population in ONE persistent launch (the per-member self-play slices of ADAP's simultaneous trainer and of
+ * XD's conventions, train/ADAP/simultaneous.py, train/XD/serial.py): the worlds [128 s, 128 s + 128) are played by weight
+ * set slice_policy[s] on both seats, actor + critic, hidden 64.  slice_policy: DEVICE int32 [N / 128], every entry in
+ * [0, n_policies) of the handle (not checked: the table stays on the device; an entry out of range reads outside the
+ * weights, as with the tile_policy tables of the other entry points).  The same buffers, bit
+ * for bit, as ocb_rollout_policy(tile_policy = slice_policy ++ slice_policy, values != NULL) — same sampling counters, same
+ * env transitions, same bootstrap values[T].  obs_slab, actions and values are required (OCB_ERR_INVALID_ARG otherwise, and
+ * when N is not a multiple of 128); obs_slab[0] is written by the kernel.  OCB_ERR_UNSUPPORTED for hidden 512 and for
+ * layouts the fused kernel does not take — callers then use ocb_rollout_policy. */
+int ocb_rollout_population_fused(ocb_env* env, ocb_policy* pol, int T, const int32_t* slice_policy, int8_t* obs_slab,
+                                 int32_t* actions, float* logp, float* values, int32_t* reward, int32_t* done,
+                                 int deterministic, uint64_t seed, void* stream);
+
 /* Diagnostic: ocb_rollout_policy_fused through the instrumented build of the kernel (synchronous, sampled
  * actions).  h_trace (HOST int64 [n_steps][64]) receives clock64 stamps of CTA 0 for steps u0 .. u0+n_steps-1;
  * event indices are listed at trace_ev in csrc/policy_kernels.cu (env / loader / MMA issue / epilogue hand-offs).
