@@ -5,32 +5,32 @@
 //   obs int8 [M, W, H, C=20] -> Conv3x3(20->32) -> ReLU -> FC((W-2)(H-2)*32 -> 64) -> ReLU
 //   -> FC(64->64) -> ReLU -> head (6 logits, orthogonal gain 0.01 | 1 value).
 //
-// One persistent, warp-specialised kernel runs BOTH networks (even CTAs the actor, odd CTAs the
-// critic); a work unit is (tile of 128 observation rows, network):
+// One persistent, warp-specialised kernel (policy_pair_kernel, one CTA per SM) runs BOTH networks of
+// every tile of 128 observation rows in the same CTA:
 //   * loader warps (2 groups of 4, alternating grid columns): coalesced loads of one grid column
 //     of the tile ([128 rows] x H cells x 20 B, software-prefetched in registers), transposed
 //     through a small staging buffer into per-cell [128 x 16] bf16 K-major operand blocks held in
 //     a ring of 4 grid columns (int8 -> bf16 is one PRMT + one HADD2.BF16 per channel pair).  The
 //     convolution needs NO im2col: for output position (ox, oy) the k-slice of window cell
 //     (dx, dy) is the block of cell (ox+dx, oy+dy), so the conv is 9 x (hi, lo) tcgen05.mma
-//     (M128 N32 K16) per position pointing at different blocks; the 5 static terrain channels
-//     are folded into a per-position bias on the host;
-//   * one MMA thread issues every tcgen05.mma; accumulators live in TMEM (conv: 4 stages x 32
-//     columns, FC1 and FC2: 2 x 64 columns each, double-buffered across units) and the issue
-//     order keeps the conv up to 3 positions ahead of the FC1 partial sums so the tensor pipe
-//     has work while the epilogue warps run;
-//   * epilogue warps (2 groups of 4, alternating items == A-operand ring stages): tcgen05.ld a
-//     conv position, bias + ReLU, split into bf16 hi + lo and store it as the A operand of the
-//     FC1 partial product of that position (2-stage ring); FC2 flows through the same ring as
-//     two more K=32 items fed from the FC1 accumulator; the tiny head (64 -> 6 | 1) is split by
-//     hidden halves over the two groups, softmax sampling and log-prob run in fp32 on CUDA cores;
-//   * one producer thread streams the FC weights as 8 KB chunks with cp.async.bulk
+//     per position pointing at different blocks; the 5 static terrain channels are folded into a
+//     per-position bias on the host;
+//   * two conv issuers (even / odd positions = the two accumulator stages) run one N = 64 conv
+//     for both networks, one FC issuer per network issues its FC1 partial products and FC2;
+//     accumulators live in TMEM (see the pair kernel's section below);
+//   * epilogue warps (2 groups of 4, group g = network g): tcgen05.ld a conv position, bias + ReLU,
+//     split into bf16 hi + lo and store it as the A operand of the FC1 partial product of that
+//     position; FC2 flows through the same A stage as two more K=32 items fed from the FC1
+//     accumulator; the tiny head (64 -> 6 | 1), softmax sampling and log-prob run in fp32 on CUDA cores;
+//   * one producer thread streams the FC weights of both networks as 8 KB chunks with cp.async.bulk
 //     (global -> shared, mbarrier complete_tx) into a ring; when the whole set fits the ring
 //     the chunks stay resident and are only re-fetched when a tile selects another policy;
+//   * single mode (ocb_policy_act / ocb_policy_value): one network per tile as one stream, both
+//     epilogue groups on it, bit-identical to the two-network forward;
 //   * precision: operands are bf16 hi+lo splits (x = hi + lo, 3 products, fp32 accumulate),
 //     observations are exact in bf16, so logits agree with the fp32 reference to ~1e-5
 //     relative (the 1e-3 bar of the north star is not reachable with plain bf16 operands);
-//   * activations never touch HBM; per unit the kernel reads the tile's observations once.
+//   * activations never touch HBM; per tile the kernel reads the tile's observations once.
 // All inter-role hand-offs are mbarriers; waits are bounded spins that trap instead of hanging.
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
@@ -58,22 +58,16 @@ constexpr int kSlots = 16;     // bf16 slots per cell: channels 0-9, 16-19, 15, 
 constexpr int kK1 = 9 * kSlots;  // conv K
 constexpr int kCellCols = kSlots / 2;  // TMEM columns of one cell block
 constexpr int kColRing = 4;    // grid columns resident per CTA (3 in use by the conv + 1 being loaded)
-constexpr int kD1Stages = 4;   // conv accumulators in flight
-constexpr int kConvAhead = 3;  // conv positions issued ahead of their FC1 item (< kD1Stages, see mma_role)
 constexpr int kChunk = 8192;   // one FC weight chunk: [64 x 32] bf16 hi | lo
 constexpr int kA2Cols = 32;    // TMEM columns of one FC A-operand stage: [128 x 32] bf16 hi (16) | lo (16)
-constexpr int kMaxRing = 16;   // weight-ring slots (resident when >= chunks per unit)
 constexpr int kMaxH = 6;       // a grid column must fit one warp-wide load (5*H words <= 32)
 constexpr int kEpiWarps = 8;   // warps 0-7: two epilogue groups (group = warp / 4; TMEM lanes 32 (warp % 4) ..)
 constexpr int kLoadWarps = 8;  // warps 8-15: two loader groups
 constexpr int kWarpMma = kEpiWarps + kLoadWarps, kWarpProd = kWarpMma + 1;
 constexpr int kThreads = 32 * (kWarpProd + 1);  // 576
 constexpr int kTmemCols = 512;
-// TMEM map (32-bit columns x 128 lanes = rows of the tile): the A operands live here too, two bf16 per column
+// TMEM (32-bit columns x 128 lanes = rows of the tile): the cell blocks of the loaders start at column 0, two bf16 per column
 constexpr int kColCells = 0;    // ring of 4 grid columns x H cells x 8 columns ([128 x 16] bf16 each), <= 192
-constexpr int kColD1 = 192;     // conv accumulators, 4 stages x 32
-constexpr int kColA2 = 320;     // FC A operand, 2 stages x (hi 16 | lo 16)
-constexpr int kColD2 = 384;     // FC1 accumulator (then FC2 accumulator of the same unit), 2 units x 64
 constexpr int kSmemBudget = 227 * 1024 - 256;
 
 // packed weight blob of one network: a resident "head" followed by 8 KB FC chunks
@@ -124,9 +118,8 @@ struct PolicyParams {
     // sampling rows of a sharded env (ocb_policy_set_sampling_rows): launch row r draws from counter row
     // r + (r < rng_rows_per_seat ? rng_add0 : rng_add1); all zero = the launch row itself
     unsigned int rng_rows_per_seat, rng_add0, rng_add1;
-    int net_mask;             // 1 actor, 2 critic, 3 both (even CTAs actor, odd critic)
-    int ring;                 // weight-ring slots in shared memory
-    int pair_ring;            // same for policy_pair_kernel (chunks of both networks)
+    int net_mask;             // 1 actor, 2 critic, 3 both (hidden 512: even CTAs actor, odd critic)
+    int pair_ring;            // weight-ring slots in shared memory (chunks of both networks)
     int stage_stride;         // words per row of the loader staging buffer (odd)
     long long* prof;          // diagnostic build: [ctas][4 roles][PW_COUNT] stall cycles
     long long* trace;         // diagnostic build of the fused rollout: [trace_n steps][kTraceEvents] clock64 stamps of CTA 0
@@ -140,36 +133,10 @@ struct PolicyParams {
     int f_vt_round, f_slots, f_seat1_tiles;
 };
 
-// shared-memory carve-up (byte offsets from a 128-byte aligned base)
-struct SmemLayout {
-    int stage, head, wring, xbuf, bars, total;
-};
-__host__ __device__ inline SmemLayout smem_layout(int H, int npos, int ring, int stage_stride) {
-    SmemLayout s;
-    int o = 0;
-    s.stage = o, o += al128(kLoadWarps * 32 * stage_stride * 4);
-    s.head = o, o += blob_layout(npos).head_bytes;
-    s.wring = o, o += ring * kChunk;
-    s.xbuf = o, o += 2 * kRows * 8 * 4;  // head partial sums of epilogue group 1, by unit parity
-    s.bars = o, o += 512;
-    s.total = o + 128;  // slack for aligning the dynamic base
-    return s;
-}
-
-// barrier indices inside the 512-byte barrier block (8 bytes each); [60] holds the TMEM base
+// barrier indices (8 bytes each) of loader_role's grid-column ring, the same in every kernel that runs it
 enum : int {
     B_COL_FULL = 0,                      // [4]  loader -> MMA (128 arrivals)
     B_COL_EMPTY = 4,                     // [4]  MMA commit -> loader
-    B_D1_FULL = 8,                       // [4]  MMA commit -> epilogue
-    B_A2_FULL = 12,                      // [2]  epilogue -> MMA (128 arrivals)
-    B_A2_EMPTY = 14,                     // [2]  MMA commit -> epilogue
-    B_W_FULL = 16,                       // [16] bulk copy complete_tx -> MMA
-    B_W_EMPTY = 32,                      // [16] MMA commit -> producer
-    B_HEAD_FULL = 48,                    //      bulk copy -> MMA, epilogue
-    B_HEAD_EMPTY = 49,                   // [2]  by unit parity: MMA commit + 256 epilogue arrivals -> producer
-    B_D2_FULL = 51,                      //      MMA commit -> epilogue
-    B_D3_FULL = 52,                      //      MMA commit -> epilogue
-    B_COUNT = 53
 };
 
 // ---------------------------------------------------------------- PTX helpers
@@ -433,156 +400,6 @@ __device__ __forceinline__ void loader_role(long long* pw, const PolicyParams& p
     }
 }
 
-// producer: weight head (conv weights, biases, head) and the FC chunk ring
-template <bool kProf>
-__device__ __forceinline__ void producer_role(long long* pw, const PolicyParams& prm, const UnitRange ur, const BlobLayout L, uint32_t s_head,
-                                              uint32_t s_wring, uint32_t bars) {
-    const int R = prm.ring;
-    const bool resident = R >= L.chunks;
-    const int Reff = resident ? L.chunks : R;
-    uint32_t u = 0;
-    int slot = 0;
-    uint32_t round = 0;  // completed passes over the ring
-    for (int t = ur.t0; t < ur.t1; ++t, ++u) {
-        const bool chg = blob_changed(prm, t, ur.t0);
-        const uint8_t* blob = prm.blobs + ((size_t)tile_pol(prm, t) * 2 + ur.net) * prm.blob_stride;
-        if (chg) {
-            // the previous unit must be completely done with the head (conv MMAs, biases, head weights);
-            // arrivals alternate between two barriers so that a late waiter cannot alias an older phase
-            if (u > 0) mbar_wait_p<kProf>(bars + 8 * (B_HEAD_EMPTY + ((u - 1) & 1)), ((u - 1) >> 1) & 1, pw[PW_HEAD_EMPTY]);
-            if (elect_one()) {
-                mbar_arrive_expect_tx(bars + 8 * B_HEAD_FULL, (uint32_t)L.head_bytes);
-                bulk_g2s(s_head, blob, (uint32_t)L.head_bytes, bars + 8 * B_HEAD_FULL);
-            }
-            __syncwarp();
-        }
-        const bool load = !resident || chg;
-        for (int j = 0; j < L.chunks; ++j) {
-            if (round > 0) mbar_wait_p<kProf>(bars + 8 * (B_W_EMPTY + slot), (round - 1) & 1, pw[PW_W_EMPTY]);
-            if (load) {
-                if (elect_one()) {
-                    mbar_arrive_expect_tx(bars + 8 * (B_W_FULL + slot), kChunk);
-                    bulk_g2s(s_wring + slot * kChunk, blob + L.head_bytes + (size_t)j * kChunk, kChunk,
-                             bars + 8 * (B_W_FULL + slot));
-                }
-                __syncwarp();
-            }
-            if (++slot == Reff) slot = 0, ++round;
-        }
-    }
-}
-
-// MMA issuer (one thread)
-template <bool kProf>
-__device__ __forceinline__ void mma_role(long long* pw, const PolicyParams& prm, const UnitRange ur, const BlobLayout L, uint32_t tmem,
-                                         uint32_t a_head, uint32_t a_wring, uint32_t bars) {
-    const int W = prm.W, H = prm.H, PH = H - 2, npos = prm.npos;
-    const int R = prm.ring;
-    const bool resident = R >= L.chunks;
-    const int Reff = resident ? L.chunks : R;
-    const uint32_t idesc32 = make_idesc(kRows, kCo), idesc64 = make_idesc(kRows, kHid);
-    const uint32_t a_wchi = a_head + L.wc_hi, a_wclo = a_head + L.wc_lo;
-
-    // conv stream
-    int tc = ur.t0, pc = 0, ox = 0, oy = 0;
-    uint32_t gcb = 0;          // running column index of column 0 of unit tc
-    uint32_t convs = 0;        // conv positions issued
-    // item stream (FC1 positions, then the two FC2 halves of each unit)
-    int ti = ur.t0, ji = 0;
-    uint32_t fc1s = 0;         // FC1 items issued
-    uint32_t items = 0;        // items issued (A2 ring counter)
-    int slot = 0;              // weight-ring slot of the next chunk
-    uint32_t wround = 0;       // completed passes over the weight ring
-    uint32_t ui = 0;           // unit counter of the item stream
-    uint32_t head_gen = 0;     // head loads waited for so far (conv stream)
-    uint32_t w_gen = 0;        // resident mode: ring fills waited for so far (item stream)
-    bool w_loaded = false;
-
-    while (ti < ur.t1) {
-        // keep the conv ahead of the FC items, but never across a change of weights (the new head is only
-        // loaded once the previous unit has drained completely)
-        const bool conv_ok = tc < ur.t1 && (int)(convs - fc1s) < kConvAhead && (tc == ti || !blob_changed(prm, tc, ur.t0));
-        if (conv_ok) {
-            if (pc == 0 && blob_changed(prm, tc, ur.t0)) {
-                mbar_wait_p<kProf>(bars + 8 * B_HEAD_FULL, head_gen & 1, pw[PW_HEAD_FULL]);
-                ++head_gen;
-            }
-            if (oy == 0) {  // new window column(s)
-                for (int d = (ox == 0 ? 0 : 2); d < 3; ++d) {
-                    const uint32_t g = gcb + ox + d;
-                    mbar_wait_p<kProf>(bars + 8 * (B_COL_FULL + g % kColRing), (g / kColRing) & 1, pw[PW_COL_FULL]);
-                }
-            }
-            tc_fence_after();
-            const uint32_t d1 = tmem + kColD1 + (convs % kD1Stages) * kCo;
-            const bool last = pc + 1 == npos;
-            const long long ti0 = kProf ? clock64() : 0;
-            if (elect_one()) {
-#pragma unroll
-                for (int j = 0; j < 9; ++j) {
-                    const int dx = j / 3, dy = j - dx * 3;
-                    const uint32_t ta = tmem + kColCells + (((gcb + ox + dx) % kColRing) * H + oy + dy) * kCellCols;
-                    umma_bf16_ts(d1, ta, make_desc(a_wchi + j * 256, 128, 2304), idesc32, j > 0);
-                    umma_bf16_ts(d1, ta, make_desc(a_wclo + j * 256, 128, 2304), idesc32, 1);
-                }
-                umma_commit(bars + 8 * (B_D1_FULL + convs % kD1Stages));
-                if (oy == PH - 1) {  // the window leaves column ox (and the last two columns with the last window)
-                    umma_commit(bars + 8 * (B_COL_EMPTY + (gcb + ox) % kColRing));
-                    if (ox == W - 3) {
-                        umma_commit(bars + 8 * (B_COL_EMPTY + (gcb + ox + 1) % kColRing));
-                        umma_commit(bars + 8 * (B_COL_EMPTY + (gcb + ox + 2) % kColRing));
-                    }
-                }
-                // last conv of the unit: the conv weights of the head are free once these MMAs complete
-                if (last) umma_commit(bars + 8 * (B_HEAD_EMPTY + ((uint32_t)(tc - ur.t0) & 1)));
-            }
-            __syncwarp();
-            if (kProf) pw[PW_ISSUE_CONV] += clock64() - ti0;
-            ++convs;
-            if (++oy == PH) oy = 0, ++ox;
-            if (++pc == npos) pc = 0, ox = 0, ++tc, gcb += W;
-            continue;
-        }
-        // ---- one FC item: D2 (+)= A2 x W1_j   or   D3 (+)= A2 x W2_half
-        if (ji == 0) {
-            w_loaded = !resident || blob_changed(prm, ti, ur.t0);
-            if (resident && w_loaded) ++w_gen;
-        }
-        const int a2s = items & 1;
-        mbar_wait_p<kProf>(bars + 8 * (B_A2_FULL + a2s), (items >> 1) & 1, pw[PW_A2_FULL]);
-        // the first FC2 product overwrites the FC1 accumulator: both halves must have been drained, i.e. the
-        // other epilogue group must have published item npos + 1 as well
-        if (ji == npos) mbar_wait_p<kProf>(bars + 8 * (B_A2_FULL + (a2s ^ 1)), ((items + 1) >> 1) & 1, pw[PW_A2_FULL]);
-        if (w_loaded) mbar_wait_p<kProf>(bars + 8 * (B_W_FULL + slot), resident ? ((w_gen - 1) & 1) : (wround & 1), pw[PW_W_FULL]);
-        tc_fence_after();
-        // FC2 accumulates into the columns of the (already drained) FC1 accumulator of the same unit
-        const uint32_t dst = tmem + kColD2 + (ui & 1) * kHid;
-        const bool first = (ji == 0 || ji == npos);
-        const uint32_t a_hi = tmem + kColA2 + a2s * kA2Cols, a_lo = a_hi + 16;
-        const uint32_t b_hi = a_wring + slot * kChunk, b_lo = b_hi + 4096;
-        const long long tf0 = kProf ? clock64() : 0;
-        if (elect_one()) {
-#pragma unroll
-            for (int ks = 0; ks < 2; ++ks) {
-                const uint64_t bhi = make_desc(b_hi + ks * 256, 128, 512), blo = make_desc(b_lo + ks * 256, 128, 512);
-                umma_bf16_ts(dst, a_hi + ks * 8, bhi, idesc64, (!first || ks != 0) ? 1u : 0u);
-                umma_bf16_ts(dst, a_hi + ks * 8, blo, idesc64, 1);
-                umma_bf16_ts(dst, a_lo + ks * 8, bhi, idesc64, 1);
-            }
-            umma_commit(bars + 8 * (B_A2_EMPTY + a2s));
-            umma_commit(bars + 8 * (B_W_EMPTY + slot));
-            if (ji == npos - 1) umma_commit(bars + 8 * B_D2_FULL);
-            if (ji == npos + 1) umma_commit(bars + 8 * B_D3_FULL);
-        }
-        __syncwarp();
-        if (kProf) pw[PW_ISSUE_FC] += clock64() - tf0;
-        ++items;
-        if (++slot == Reff) slot = 0, ++wround;
-        if (ji < npos) ++fc1s;
-        if (++ji == npos + 2) ji = 0, ++ti, ++ui;
-    }
-}
-
 // actor outputs of one row: raw logits, sampled (or arg-max) action and its log-prob
 // FixedCategorical(logits): sample / mode and log-prob (train/MAPPO/utils/distributions.py:14-28)
 // `store` indexes the output arrays, `rng_row` keys the sampling counter (they differ in the fused
@@ -686,165 +503,8 @@ __device__ __forceinline__ void head_accumulate(int net, const float (&v)[32], c
     }
 }
 
-// epilogue: TMEM -> bias/ReLU -> bf16 hi/lo A operand; head, sampling and outputs.  Two groups of four
-// warps: group g owns stage g of the A-operand ring, i.e. every other item of the CTA's item stream
-// (items of a unit: npos conv positions, then the two K halves of FC2's input).
-template <bool kProf>
-__device__ __forceinline__ void epilogue_role(long long* pw, const PolicyParams& prm, const UnitRange ur, const BlobLayout L, uint32_t tmem,
-                                              const uint8_t* s_head, float* s_xbuf, uint32_t bars) {
-    const int warp = threadIdx.x >> 5, eg = warp >> 2, trow_id = (warp & 3) * 32 + (threadIdx.x & 31);
-    const int npos = prm.npos;
-    const uint32_t trow = tmem + ((uint32_t)((warp & 3) * 32) << 16);  // this warp's 32 TMEM lanes
-    const float* s_bias1 = reinterpret_cast<const float*>(s_head + L.bias1);
-    const float* s_b1 = reinterpret_cast<const float*>(s_head + L.b1);
-    const float* s_b2 = reinterpret_cast<const float*>(s_head + L.b2);
-    const float* s_wh = reinterpret_cast<const float*>(s_head + L.wh);
-    const float* s_bh = reinterpret_cast<const float*>(s_head + L.bh);
-    unsigned long long offset = prm.offset;
-    if (prm.d_offset != nullptr) offset += *prm.d_offset;
-
-    uint32_t u = 0, head_gen = 0;
-    for (int t = ur.t0; t < ur.t1; ++t, ++u) {
-        if (blob_changed(prm, t, ur.t0)) {
-            mbar_wait_p<kProf>(bars + 8 * B_HEAD_FULL, head_gen & 1, pw[PW_HEAD_FULL]);
-            ++head_gen;
-        }
-        const uint32_t item0 = u * (uint32_t)(npos + 2);
-        for (int j = (int)((item0 ^ (uint32_t)eg) & 1u); j < npos + 2; j += 2) {
-            const uint32_t item = item0 + (uint32_t)j;  // item & 1 == eg: the ring stage of this group
-            float v[32];
-            const float* bias;
-            if (j < npos) {
-                const uint32_t d1c = u * (uint32_t)npos + (uint32_t)j;
-                const int st = d1c % kD1Stages;
-                mbar_wait_p<kProf>(bars + 8 * (B_D1_FULL + st), (d1c / kD1Stages) & 1, pw[PW_D1_FULL]);
-                tc_fence_after();
-                tmem_ld32(trow + kColD1 + st * kCo, v);
-                bias = s_bias1 + j * kCo;
-            } else {
-                mbar_wait_p<kProf>(bars + 8 * B_D2_FULL, u & 1, pw[PW_D2_FULL]);
-                tc_fence_after();
-                tmem_ld32(trow + kColD2 + (u & 1) * kHid + (j - npos) * 32, v);
-                bias = s_b1 + (j - npos) * 32;
-            }
-#pragma unroll
-            for (int i = 0; i < 32; ++i) v[i] = fmaxf(v[i] + bias[i], 0.0f);
-            if (item >= 2) {
-                mbar_wait_p<kProf>(bars + 8 * (B_A2_EMPTY + eg), ((item >> 1) - 1) & 1, pw[PW_A2_EMPTY]);
-                tc_fence_after();
-            }
-            uint32_t hi[16], lo[16];
-#pragma unroll
-            for (int i = 0; i < 16; ++i) split2(v[2 * i], v[2 * i + 1], hi[i], lo[i]);
-            tmem_st16(trow + kColA2 + eg * kA2Cols, hi);
-            tmem_st16(trow + kColA2 + eg * kA2Cols + 16, lo);
-            tmem_st_wait();
-            tc_fence_before();
-            mbar_arrive(bars + 8 * (B_A2_FULL + eg));
-        }
-
-        // ---- FC2 epilogue + head (fp32 on CUDA cores): group g covers hidden units 32 g .. 32 g + 31
-        float head[6];
-#pragma unroll
-        for (int a = 0; a < 6; ++a) head[a] = eg == 0 ? s_bh[a] : 0.0f;
-        mbar_wait_p<kProf>(bars + 8 * B_D3_FULL, u & 1, pw[PW_D3_FULL]);
-        tc_fence_after();
-        {
-            float v[32];
-            tmem_ld32(trow + kColD2 + (u & 1) * kHid + eg * 32, v);
-            head_accumulate(ur.net, v, s_b2 + eg * 32, s_wh, eg * 32, head);
-        }
-        tc_fence_before();
-        mbar_arrive(bars + 8 * (B_HEAD_EMPTY + (u & 1)));  // done with the head block of this unit
-
-        // group 1 hands its partial sums to group 0 (same rows: warps w and w + 4), double-buffered by unit parity
-        float* xrow = s_xbuf + ((u & 1) * kRows + trow_id) * 8;
-        if (eg == 1) {
-            *reinterpret_cast<float4*>(xrow) = make_float4(head[0], head[1], head[2], head[3]);
-            *reinterpret_cast<float2*>(xrow + 4) = make_float2(head[4], head[5]);
-        }
-        asm volatile("bar.sync %0, 64;" ::"r"(1 + (warp & 3)) : "memory");
-        if (eg == 1) continue;
-        {
-            const float4 x0 = *reinterpret_cast<const float4*>(xrow);
-            const float2 x1 = *reinterpret_cast<const float2*>(xrow + 4);
-            head[0] += x0.x, head[1] += x0.y, head[2] += x0.z, head[3] += x0.w, head[4] += x1.x, head[5] += x1.y;
-        }
-
-        const long long row = (long long)t * kRows + trow_id;
-        if (row < prm.M) {
-            if (ur.net == 1) {
-                if (prm.values) prm.values[row] = head[0];
-            } else {
-                emit_actor_row(prm, row, (uint32_t)row, head, offset);
-            }
-        }
-    }
-}
-
-// ---------------------------------------------------------------- the kernel
-template <bool kProf>
-__global__ void __launch_bounds__(kThreads, 1) policy_fwd_kernel(const PolicyParams prm) {
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = smem_raw + ((128u - (smem_addr(smem_raw) & 127u)) & 127u);
-    const int tid = threadIdx.x, warp = tid >> 5;
-    const BlobLayout L = blob_layout(prm.npos);
-    const SmemLayout sl = smem_layout(prm.H, prm.npos, prm.ring, prm.stage_stride);
-    uint32_t* s_stage = reinterpret_cast<uint32_t*>(smem + sl.stage);
-    uint8_t* s_head = smem + sl.head;
-    uint8_t* s_wring = smem + sl.wring;
-    float* s_xbuf = reinterpret_cast<float*>(smem + sl.xbuf);
-    uint64_t* s_bars = reinterpret_cast<uint64_t*>(smem + sl.bars);
-    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(s_bars + 60);
-    const uint32_t bars = smem_addr(s_bars);
-
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_addr(s_tmem)),
-                     "r"((uint32_t)kTmemCols)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    if (tid == 32) {
-        for (int i = 0; i < B_COUNT; ++i) {
-            uint32_t count = 1;
-            if ((i >= B_COL_FULL && i < B_COL_FULL + 4) || (i >= B_A2_FULL && i < B_A2_FULL + 2)) count = 128;
-            if (i >= B_HEAD_EMPTY && i < B_HEAD_EMPTY + 2) count = 32 * kEpiWarps + 1;
-            mbar_init(bars + 8 * i, count);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *s_tmem;
-    const UnitRange ur = my_units(prm);
-
-    long long pw[kProf ? PW_COUNT : 1] = {};
-    const long long t_begin = kProf ? clock64() : 0;
-    if (warp < kEpiWarps) {
-        epilogue_role<kProf>(pw, prm, ur, L, tmem, s_head, s_xbuf, bars);
-    } else if (warp < kWarpMma) {
-        loader_role<kProf>(pw, prm, ur, tmem, s_stage, bars);
-    } else if (warp == kWarpMma) {  // whole warp runs the control flow, one elected lane issues
-        mma_role<kProf>(pw, prm, ur, L, tmem, smem_addr(s_head), smem_addr(s_wring), bars);
-    } else {
-        producer_role<kProf>(pw, prm, ur, L, smem_addr(s_head), smem_addr(s_wring), bars);
-    }
-    if (kProf && prm.prof != nullptr &&
-        (tid == 0 || tid == 32 * kEpiWarps || tid == 32 * kWarpMma || tid == 32 * kWarpProd)) {
-        pw[PW_TOTAL] = clock64() - t_begin;
-        const int role = tid == 0 ? 0 : tid == 32 * kEpiWarps ? 1 : tid == 32 * kWarpMma ? 2 : 3;  // epilogue, loader, MMA, producer
-        for (int i = 0; i < PW_COUNT; ++i) prm.prof[((size_t)blockIdx.x * 4 + role) * PW_COUNT + i] = pw[i];
-    }
-    __syncwarp();
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((uint32_t)kTmemCols) : "memory");
-}
-
 // ================================================================ pair kernel: both networks of a tile in ONE CTA
-// The fused actor+critic forward (ocb_policy_forward / ocb_rollout_policy) runs this variant.  A work
+// Every hidden-64 forward runs this kernel (the single-network calls in its single mode, below).  A work
 // unit is a tile of 128 rows; the CTA computes the actor AND the critic for it:
 //   * the observation columns are loaded and converted once for both networks (loader_role above);
 //   * the conv is ONE accumulate of N = 64 (actor channels 0-31 | critic channels 32-63): the two
@@ -854,7 +514,7 @@ __global__ void __launch_bounds__(kThreads, 1) policy_fwd_kernel(const PolicyPar
 //     accumulate into the (by then drained) conv accumulator stage g; the whole head of network g is
 //     evaluated by group g (no cross-group reduction);
 //   * TMEM: cells 0-191 | conv accumulators 2 x 64 (later D3 of net 0 / net 1) | A stage 2 x 32 | D2 2 x 64.
-// Compared with the (tile, network) units of policy_fwd_kernel this doubles the work in flight per SM
+// Compared with one network per CTA this doubles the work in flight per SM
 // (the pipeline is latency-bound: every hand-off is an mbarrier round trip), halves the loader work
 // and the number of conv MMA instructions, and lets 128 tiles (config 4: 8,192 worlds) run as ONE wave.
 constexpr int kPColD1 = 192;   // conv accumulators: stage s at + 64 s (actor 32 | critic 32); D3 of net g = stage g
@@ -1515,12 +1175,9 @@ void put_split(uint8_t* hi, uint8_t* lo, size_t off, float w) {
 struct ocb_policy {
     int device;
     int W, H, S, SC, C, npos, n_policies;
-    int sm_count, ring, stage_stride;
-    size_t smem_bytes;
-    int pair_ring;            // 0: the pair kernel is not usable for this layout
+    int sm_count, stage_stride;
+    int pair_ring;            // weight-ring slots of policy_pair_kernel (0 for hidden 512 and the generic kernel)
     size_t pair_smem_bytes;
-    int use_pair;             // run ocb_policy_forward through policy_pair_kernel (env OCB_POLICY_PAIR=0 disables)
-    int use_single;           // ... and the single-network calls through its one-stream mode (env OCB_POLICY_SINGLE=0: policy_fwd_kernel)
     std::vector<uint8_t> terrain;
     BlobLayout L;
     uint8_t* d_blobs;
@@ -1604,7 +1261,7 @@ extern "C" int ocb_policy_create(const ocb_config* cfg, int device, int hidden, 
     p->generic = generic ? 1 : 0;
     p->npos = (p->W - 2) * (p->H - 2), p->n_policies = n_policies, p->calls = 0, p->d_blobs = nullptr;
     p->hidden = hidden, p->d_scratch = nullptr, p->scratch_tiles = 0, p->L5 = blob5_layout(p->npos);
-    p->ring = 0, p->smem_bytes = 0, p->pair_ring = 0, p->pair_smem_bytes = 0, p->use_pair = 0, p->use_single = 0;
+    p->pair_ring = 0, p->pair_smem_bytes = 0;
     p->terrain.assign(cfg->terrain, cfg->terrain + p->S);
     p->L = blob_layout(p->npos);
     p->stage_stride = (5 * p->H) | 1;
@@ -1615,30 +1272,17 @@ extern "C" int ocb_policy_create(const ocb_config* cfg, int device, int hidden, 
             return fail(OCB_ERR_UNSUPPORTED, "layout too large for the generic policy kernel (%d x %d)", cfg->width, cfg->height);
         }
     } else if (hidden == kHid) {
-    // weight ring: as many 8 KB chunks as fit; all of them (resident weights) when possible
-    const int fixed = smem_layout(p->H, p->npos, 0, p->stage_stride).total;
-    int ring = (kSmemBudget - fixed) / kChunk;
-    if (ring > kMaxRing) ring = kMaxRing;
-    if (ring > p->L.chunks) ring = p->L.chunks;
-    if (ring < 2) {
-        delete p;
-        return fail(OCB_ERR_UNSUPPORTED, "layout too large for the fused policy kernel (%d x %d)", cfg->width, cfg->height);
-    }
-    p->ring = ring;
-    p->smem_bytes = (size_t)smem_layout(p->H, p->npos, ring, p->stage_stride).total;
-    // pair kernel (both networks per CTA): ring over the chunks of both networks
-    {
-        const int pfixed = pair_smem_layout(p->npos, 0, p->stage_stride).total;
-        int pring = (kSmemBudget - pfixed) / kChunk;
-        if (pring > kPMaxRing) pring = kPMaxRing;
-        if (pring > 2 * p->L.chunks) pring = 2 * p->L.chunks;
-        p->pair_ring = pring >= 4 ? pring : 0;
-        p->pair_smem_bytes = p->pair_ring ? (size_t)pair_smem_layout(p->npos, p->pair_ring, p->stage_stride).total : 0;
-        const char* e = getenv("OCB_POLICY_PAIR");
-        p->use_pair = p->pair_ring != 0 && !(e != nullptr && e[0] == '0');
-        const char* e1 = getenv("OCB_POLICY_SINGLE");
-        p->use_single = !(e1 != nullptr && e1[0] == '0');
-    }
+        // weight ring over the FC chunks of both networks: as many 8 KB slots as fit; all of them (resident weights) when
+        // possible.  Every layout with H <= kMaxH and at most OCB_MAX_CELLS cells leaves room for 8 or more.
+        int ring = (kSmemBudget - pair_smem_layout(p->npos, 0, p->stage_stride).total) / kChunk;
+        if (ring > kPMaxRing) ring = kPMaxRing;
+        if (ring > 2 * p->L.chunks) ring = 2 * p->L.chunks;
+        if (ring < 4) {
+            delete p;
+            return fail(OCB_ERR_UNSUPPORTED, "layout too large for the fused policy kernel (%d x %d)", cfg->width, cfg->height);
+        }
+        p->pair_ring = ring;
+        p->pair_smem_bytes = (size_t)pair_smem_layout(p->npos, ring, p->stage_stride).total;
     } else if (c5_smem_layout(p->npos, p->stage_stride).total > kSmemBudget + 128) {
         delete p;
         return fail(OCB_ERR_UNSUPPORTED, "layout too large for the hidden-512 conv kernel (%d x %d)", cfg->width, cfg->height);
@@ -1657,8 +1301,6 @@ extern "C" int ocb_policy_create(const ocb_config* cfg, int device, int hidden, 
     }
     // the opt-in limit is per function, not per handle: always raise it to the full budget
     const int smem_max = kSmemBudget + 128;
-    if (err == cudaSuccess) err = cudaFuncSetAttribute(policy_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
-    if (err == cudaSuccess) err = cudaFuncSetAttribute(policy_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(policy_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(policy_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
@@ -1924,8 +1566,7 @@ static int policy_launch(ocb_policy* p, int net_mask, const int8_t* obs, int M, 
     prm.deterministic = deterministic, prm.seed = seed, prm.offset = offset;
     prm.rng_rows_per_seat = p->rng_rows_per_seat, prm.rng_add0 = p->rng_add0, prm.rng_add1 = p->rng_add1;
     prm.d_offset = reinterpret_cast<const unsigned long long*>(d_offset);
-    prm.net_mask = net_mask, prm.ring = p->ring, prm.stage_stride = p->stage_stride;
-    prm.pair_ring = p->pair_ring;
+    prm.net_mask = net_mask, prm.pair_ring = p->pair_ring, prm.stage_stride = p->stage_stride;
     prm.prof = prof;
     if (ev != nullptr) prm.row_index = ev->row_index, prm.given_actions = ev->given_actions, prm.entropy = ev->entropy;
     if (p->generic) {
@@ -1949,29 +1590,14 @@ static int policy_launch(ocb_policy* p, int net_mask, const int8_t* obs, int M, 
         if (ctas_out) *ctas_out = 0;
         return policy_launch512(p, prm, (cudaStream_t)stream);
     }
-    // persistent grid: one CTA per SM
-    int ctas;
-    if (p->use_pair && (net_mask == 3 || p->use_single)) {  // both networks of a tile in one CTA, or the one asked for as one stream
-        prm.single = net_mask == 3 ? 0 : net_mask;
-        ctas = prm.tiles < p->sm_count ? prm.tiles : p->sm_count;
-        if (ctas_out) *ctas_out = ctas;
-        if (prof != nullptr)
-            policy_pair_kernel<true><<<ctas, kPThreads, p->pair_smem_bytes, (cudaStream_t)stream>>>(prm);
-        else
-            policy_pair_kernel<false><<<ctas, kPThreads, p->pair_smem_bytes, (cudaStream_t)stream>>>(prm);
-    } else {
-        if (net_mask == 3) {  // (tile, network) units: even CTAs run the actor, odd ones the critic
-            const int per_net = prm.tiles < p->sm_count / 2 ? prm.tiles : p->sm_count / 2;
-            ctas = 2 * per_net;
-        } else {
-            ctas = prm.tiles < p->sm_count ? prm.tiles : p->sm_count;
-        }
-        if (ctas_out) *ctas_out = ctas;
-        if (prof != nullptr)
-            policy_fwd_kernel<true><<<ctas, kThreads, p->smem_bytes, (cudaStream_t)stream>>>(prm);
-        else
-            policy_fwd_kernel<false><<<ctas, kThreads, p->smem_bytes, (cudaStream_t)stream>>>(prm);
-    }
+    // persistent grid, one CTA per SM: both networks of a tile in one CTA, or the one asked for as one stream
+    prm.single = net_mask == 3 ? 0 : net_mask;
+    const int ctas = prm.tiles < p->sm_count ? prm.tiles : p->sm_count;
+    if (ctas_out) *ctas_out = ctas;
+    if (prof != nullptr)
+        policy_pair_kernel<true><<<ctas, kPThreads, p->pair_smem_bytes, (cudaStream_t)stream>>>(prm);
+    else
+        policy_pair_kernel<false><<<ctas, kPThreads, p->pair_smem_bytes, (cudaStream_t)stream>>>(prm);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return fail(OCB_ERR_CUDA, "policy kernel launch failed: %s", cudaGetErrorString(err));
     p->calls += 1;
@@ -2023,9 +1649,9 @@ extern "C" int ocb_policy_set_sampling_rows(ocb_policy* p, uint32_t rows_per_sea
 
 extern "C" int ocb_policy_info(const ocb_policy* p, int* ring_slots, int* chunks_per_unit, int* smem_bytes) {
     if (p == nullptr) return fail(OCB_ERR_INVALID_ARG, "policy is NULL");
-    if (ring_slots) *ring_slots = p->ring;
-    if (chunks_per_unit) *chunks_per_unit = p->L.chunks;
-    if (smem_bytes) *smem_bytes = (int)p->smem_bytes;
+    if (ring_slots) *ring_slots = p->pair_ring;
+    if (chunks_per_unit) *chunks_per_unit = 2 * p->L.chunks;
+    if (smem_bytes) *smem_bytes = (int)p->pair_smem_bytes;
     return OCB_OK;
 }
 

@@ -219,7 +219,8 @@ int ocb_policy_act_ex(ocb_policy* pol, const int8_t* obs, int M, const int32_t* 
 int ocb_policy_value(ocb_policy* pol, const int8_t* obs, int M, const int32_t* tile_policy, float* values,
                      void* stream);
 
-/* both networks in ONE launch (even CTAs run the actor, odd CTAs the critic): everything
+/* both networks in ONE launch (hidden 64: one CTA runs both networks of a 128-row tile; hidden 512:
+ * even CTAs run the actor, odd CTAs the critic): everything
  * ocb_policy_act and ocb_policy_value write; values is required.  d_offset (DEVICE pointer, may
  * be NULL) is added to `offset` on the device, so a CUDA graph that replays this launch samples
  * with a fresh counter (pass ocb_step_counter_device(env)). */
@@ -233,8 +234,9 @@ int ocb_policy_forward(ocb_policy* pol, const int8_t* obs, int M, const int32_t*
  * is bit-identical to the single-GPU one.  Applies to every later sampling launch of this handle; (0, 0, 0) restores
  * the default.  Not in the reference (its sampling is torch's global generator, train/MAPPO/utils/distributions.py:14-20). */
 int ocb_policy_set_sampling_rows(ocb_policy* pol, uint32_t rows_per_seat, uint32_t add_seat0, uint32_t add_seat1);
-/* launch shape in effect: weight-ring slots in shared memory, FC weight chunks per (tile, network)
- * unit (ring >= chunks means the weights stay resident), dynamic shared memory per CTA */
+/* launch shape of the hidden-64 forward: weight-ring slots in shared memory, FC weight chunks of
+ * both networks per tile (ring >= chunks means the weights stay resident), dynamic shared memory
+ * per CTA; ring and shared memory are 0 for hidden 512 and for the generic kernel */
 int ocb_policy_info(const ocb_policy* pol, int* ring_slots, int* chunks_per_unit, int* smem_bytes);
 /* pre-size the handle's internal activation scratch (hidden 512 only) for forwards of up to M rows:
  * required before a forward of a new, larger M is captured into a CUDA graph */

@@ -43,14 +43,11 @@ def main():
                                                            prof.ctypes.data_as(ctypes.c_void_p), 256))
     p = prof[:ctas]
     print(json.dumps({"layout": args.layout, "ctas": ctas, "info": pol.info()}))
-    pair = os.environ.get("OCB_POLICY_PAIR", "1") != "0"  # pair kernel: every CTA runs both networks
-    for net, nm in (((0, "all CTAs (pair kernel; epilogue = actor group)"),) if pair else ((0, "actor CTAs"), (1, "critic CTAs"))):
-        sel = p if pair else p[net::2]
-        print(nm, "mean cycles over", len(sel), "CTAs")
-        for r, rn in enumerate(ROLES):
-            m = sel[:, r, :].mean(axis=0)
-            parts = ", ".join("%s %d" % (NAMES[i], m[i]) for i in range(1, len(NAMES)) if m[i] > 0)
-            print("  %-9s total %7d  busy %7d | %s" % (rn, m[0], m[0] - m[1:NWAIT].sum(), parts))
+    print("all CTAs (pair kernel; epilogue = actor group)", "mean cycles over", len(p), "CTAs")
+    for r, rn in enumerate(ROLES):
+        m = p[:, r, :].mean(axis=0)
+        parts = ", ".join("%s %d" % (NAMES[i], m[i]) for i in range(1, len(NAMES)) if m[i] > 0)
+        print("  %-9s total %7d  busy %7d | %s" % (rn, m[0], m[0] - m[1:NWAIT].sum(), parts))
 
 
 if __name__ == "__main__":
