@@ -73,6 +73,7 @@ PROTOTYPES = {
     "ocb_rollout_fused_debug_trace": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _vp, _i, _i]),
     "ocb_rollout_mixed_scratch_bytes": (_sz, [_vp]),
     "ocb_rollout_mixed": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _u64, _u64, _vp, _sz, _vp]),
+    "ocb_rollout_mixed_fused": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _u64, _u64, _vp]),
     "ocb_compute_returns": (_i, [_i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "ocb_compute_returns_dev": (_i, [_i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "ocb_normalize_advantages": (_i, [_i, _vp, _sz, _vp, _vp]),

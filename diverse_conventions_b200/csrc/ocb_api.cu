@@ -878,3 +878,51 @@ extern "C" int ocb_rollout_mixed(ocb_env* e, ocb_policy* pol, int L, int main_po
     return OCB_OK;
 #undef OCB_CU
 }
+
+// The collection of ocb_rollout_mixed in one persistent launch (rollout_fused.cuh, kMix): both actors in the pipeline, the
+// per-row switch and the record of the forced worlds on the device.  Then main's critic over obs_buf[:L] in one value launch
+// (every (t < L, seat, world) cell is recorded exactly once, so that is the per-step path's values[:L], bit for bit), and
+// slot L as ocb_rollout_mixed leaves it.
+extern "C" int ocb_rollout_mixed_fused(ocb_env* e, ocb_policy* pol, int L, int main_policy, int partner_policy, int8_t* obs_buf,
+                                       int32_t* actions, float* logp, float* values, int32_t* reward, int32_t* done,
+                                       int deterministic, uint64_t seed, uint64_t mix_seed, void* stream) {
+    if (e == nullptr || pol == nullptr) return fail(OCB_ERR_INVALID_ARG, "NULL handle");
+    if (obs_buf == nullptr || actions == nullptr) return fail(OCB_ERR_INVALID_ARG, "obs_buf and actions are required");
+    if (e->P != 2) return fail(OCB_ERR_UNSUPPORTED, "the policy rollout supports 2 players");
+    if (L < 2) return fail(OCB_ERR_INVALID_ARG, "L must be >= 2");
+    if (e->N % (L - 1) != 0)
+        return fail(OCB_ERR_INVALID_ARG, "the env must hold a multiple of L - 1 = %d worlds (got %d)", L - 1, e->N);
+    const int sets = ocb_policy_num_sets(pol);
+    if (main_policy < 0 || main_policy >= sets || partner_policy < 0 || partner_policy >= sets)
+        return fail(OCB_ERR_INVALID_ARG, "policy index out of range (the handle holds %d sets)", sets);
+    // the kernel stores observation rows as 4-byte words and the value pass reads them so: reject before anything runs
+    if ((reinterpret_cast<uintptr_t>(obs_buf) & 3u) != 0) return fail(OCB_ERR_INVALID_ARG, "obs_buf must be 4-byte aligned");
+    DeviceGuard guard(e->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t PN = (size_t)e->P * e->N, obs_step = PN * (size_t)e->SC;
+    RolloutParams p = base_params(e);
+    FusedMixArgs mix;
+    mix.L = L, mix.partner_policy = partner_policy, mix.mix_seed = mix_seed;
+    mix.partner_seed = seed ^ 0x9E3779B97F4A7C15ull;  // the partner's sampling key of ocb_rollout_mixed
+    int rc = ocb_policy_rollout_fused_launch(pol, main_policy, nullptr, false, p, e->h_tables.W, e->h_tables.H, 2 * L, obs_buf, actions,
+                                             logp, nullptr, reward, done, deterministic, seed,
+                                             reinterpret_cast<const uint64_t*>(e->d_step_counter),
+                                             reinterpret_cast<uint64_t*>(e->d_step_counter), stream, nullptr, 0, 0, &mix);
+    if (rc != OCB_OK) return rc;
+    if (stream_capturing(stream))
+        e->count_stale = true;
+    else
+        e->step_count += (uint64_t)(2 * L);
+    if (values != nullptr) {
+        rc = ocb_policy_value_of(pol, main_policy, obs_buf, (int)((size_t)L * PN), values, stream);
+        if (rc != OCB_OK) return rc;
+    }
+    cudaError_t err = cudaMemsetAsync(obs_buf + (size_t)L * obs_step, 0, obs_step, st);
+    if (err == cudaSuccess && values != nullptr)
+        err = launch_fill_f32(values + (size_t)L * PN, PN, ocb_policy_zero_obs_value(pol, main_policy), st);
+    if (err != cudaSuccess) {
+        cudaGetLastError();
+        return fail(OCB_ERR_CUDA, "ocb_rollout_mixed_fused: %s", cudaGetErrorString(err));
+    }
+    return OCB_OK;
+}

@@ -44,6 +44,7 @@
 #include "api_common.h"
 #include "oc_core.cuh"
 #include "oc_device.cuh"
+#include "mixed_schedule.h"
 #include "ocb.h"
 #include "policy_internal.h"
 
@@ -566,9 +567,11 @@ __host__ __device__ inline PairSmemLayout pair_smem_layout(int npos, int ring, i
 }
 
 // kPop (population self-play in the fused rollout): the two streams are the actor and critic of the slice's weight set
-template <bool kProf, bool kPop = false>
+// kMix (mixed play in the fused rollout): stream 0 is the actor at prm.blobs, stream 1 the actor at `mix_partner`
+template <bool kProf, bool kPop = false, bool kMix = false>
 __device__ __forceinline__ void pair_producer_role(long long* pw, const PolicyParams& prm, int t0, int t1, const BlobLayout L,
-                                                   uint32_t s_head, uint32_t s_wring, uint32_t bars) {
+                                                   uint32_t s_head, uint32_t s_wring, uint32_t bars,
+                                                   const uint8_t* mix_partner = nullptr) {
     const int nets = prm.single ? 1 : 2;  // single mode: the one network takes the actor's places (stream 0, ring slots 0, 1, ...)
     const int R = prm.pair_ring, nch = nets * L.chunks;
     const bool resident = R >= nch;
@@ -583,7 +586,8 @@ __device__ __forceinline__ void pair_producer_role(long long* pw, const PolicyPa
         const int tp = tile_pol(prm, t);
         const bool cross = prm.f_vt_round != 0 && prm.tile_policy != nullptr;  // both streams are actors (of two policies)
         const uint8_t* blob_a = prm.blobs + ((size_t)(cross ? (tp & 0xFFFF) : tp) * 2 + (prm.single == 2 ? 1 : 0)) * prm.blob_stride;
-        const uint8_t* blob_c = cross && !kPop ? prm.blobs + (size_t)(tp >> 16) * 2 * prm.blob_stride : blob_a + prm.blob_stride;
+        const uint8_t* blob_c = kMix ? mix_partner
+                                     : cross && !kPop ? prm.blobs + (size_t)(tp >> 16) * 2 * prm.blob_stride : blob_a + prm.blob_stride;
         if (chg) {
             if (u > 0) mbar_wait_p<kProf>(bars + 8 * (PB_HEAD_EMPTY + ((u - 1) & 1)), ((u - 1) >> 1) & 1, pw[PW_HEAD_EMPTY]);
             if (elect_one()) {
@@ -793,7 +797,7 @@ __device__ __forceinline__ void pair_fc_role(long long* pw, const PolicyParams& 
 }
 
 // `out(t, trow_id, g, head)` consumes the head outputs of row trow_id of tile t (g = 0: six logits, g = 1: head[0] = value)
-template <bool kProf, bool kSplit, bool kPop = false, class Out>
+template <bool kProf, bool kSplit, bool kPop = false, bool kMix = false, class Out>
 __device__ __forceinline__ void pair_epilogue_role(long long* pw, const PolicyParams& prm, int t0, int t1, const BlobLayout L, uint32_t tmem,
                                                    const uint8_t* s_head, uint32_t bars, Out&& out) {
     const int warp = threadIdx.x >> 5, g = warp >> 2, trow_id = (warp & 3) * 32 + (threadIdx.x & 31);
@@ -806,8 +810,8 @@ __device__ __forceinline__ void pair_epilogue_role(long long* pw, const PolicyPa
     const float* s_wh = reinterpret_cast<const float*>(rest + L.wh);
     const float* s_bh = reinterpret_cast<const float*>(rest + L.bh);
     const uint32_t a2 = trow + kPColA2 + g * kA2Cols;
-    // head layout / outputs: 0 = actor (6 logits), 1 = critic (value); fused cross-play: two actors
-    const int net = (!kPop && prm.f_vt_round != 0 && prm.tile_policy != nullptr) ? 0 : (prm.single == 2 ? 1 : g);
+    // head layout / outputs: 0 = actor (6 logits), 1 = critic (value); fused cross-play and mixed play: two actors
+    const int net = (kMix || (!kPop && prm.f_vt_round != 0 && prm.tile_policy != nullptr)) ? 0 : (prm.single == 2 ? 1 : g);
 
     uint32_t u = 0, head_gen = 0, item = 0, d1_par = 0;  // d1_par: phase parity bit per conv accumulator stage
     int trace_vt = 0, trace_item = 0;
@@ -1312,6 +1316,8 @@ extern "C" int ocb_policy_create(const ocb_config* cfg, int device, int hidden, 
     if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, false, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, true, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, false, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, false, 1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, false, 2, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(conv512_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(gemm512_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(gemm512_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
@@ -1552,14 +1558,14 @@ struct EvalArgs {
 static int policy_launch(ocb_policy* p, int net_mask, const int8_t* obs, int M, const int32_t* tile_policy, float* logits,
                          int32_t* actions, float* logp, float* values, int deterministic, uint64_t seed, uint64_t offset,
                          const uint64_t* d_offset, void* stream, long long* prof = nullptr, int* ctas_out = nullptr,
-                         const EvalArgs* ev = nullptr) {
+                         const EvalArgs* ev = nullptr, int policy_index = 0) {
     if (p == nullptr || obs == nullptr) return fail(OCB_ERR_INVALID_ARG, "NULL argument");
     if (M < 1) return fail(OCB_ERR_INVALID_ARG, "M must be >= 1");
     if (!p->generic && (reinterpret_cast<uintptr_t>(obs) & 3u) != 0) return fail(OCB_ERR_INVALID_ARG, "obs must be 4-byte aligned");
     DeviceGuard guard(p->device);
     PolicyParams prm;
     memset(&prm, 0, sizeof(prm));
-    prm.blobs = p->d_blobs, prm.blob_stride = (size_t)p->L.total;
+    prm.blobs = p->d_blobs + (size_t)policy_index * 2 * (size_t)p->L.total, prm.blob_stride = (size_t)p->L.total;
     prm.W = p->W, prm.H = p->H, prm.S = p->S, prm.SC = p->SC, prm.npos = p->npos;
     prm.obs = obs, prm.M = M, prm.tiles = (M + kRows - 1) / kRows, prm.tile_policy = tile_policy;
     prm.logits = logits, prm.actions = actions, prm.logp = logp, prm.values = values;
@@ -1655,6 +1661,14 @@ extern "C" int ocb_policy_info(const ocb_policy* p, int* ring_slots, int* chunks
     return OCB_OK;
 }
 
+int ocb_policy_value_of(ocb_policy* p, int policy_index, const int8_t* obs, int M, float* values, void* stream) {
+    if (p == nullptr || values == nullptr) return fail(OCB_ERR_INVALID_ARG, "NULL argument");
+    if (p->generic || p->hidden != kHid) return fail(OCB_ERR_UNSUPPORTED, "ocb_policy_value_of exists for the hidden-64 tensor-core path");
+    if (policy_index < 0 || policy_index >= p->n_policies) return fail(OCB_ERR_INVALID_ARG, "policy index out of range");
+    return policy_launch(p, 2, obs, M, nullptr, nullptr, nullptr, nullptr, values, 0, 0, 0, nullptr, stream, nullptr, nullptr,
+                         nullptr, policy_index);
+}
+
 // Diagnostic: one fused forward with the instrumented build of the kernel.  h_prof (HOST, int64
 // [max_ctas][4 roles: epilogue, loader, MMA, producer][16]) receives per role the total cycles ([0])
 // and the cycles stalled on each hand-off (enum PW_* in policy_kernels.cu).  Returns the CTA count.
@@ -1690,20 +1704,30 @@ extern "C" int ocb_policy_debug_profile(ocb_policy* p, const int8_t* obs, int M,
 // output buffer optional.
 // population: tile_policy is a table by 128-world slice (int32 [N / 128], device); slice s is self-play of weight set
 // tile_policy[s] with its critic (obs_slab, actions and values required).
+// mix != nullptr: mixed play of the actors of weight sets policy_index (main) and mix->partner_policy over T = 2 L steps,
+// only the forced worlds recorded into [L, 2, N] buffers (obs_slab and actions required, no critic: values must be NULL).
 int ocb_policy_rollout_fused_launch(ocb_policy* p, int policy_index, const int32_t* tile_policy, bool population,
                                     const RolloutParams& envp, int env_w, int env_h, int T, int8_t* obs_slab, int32_t* actions,
                                     float* logp, float* values, int32_t* reward, int32_t* done, int deterministic, uint64_t seed,
                                     const uint64_t* d_offset, uint64_t* d_counter, void* stream, long long* d_trace, int trace_u0,
-                                    int trace_n) {
+                                    int trace_n, const FusedMixArgs* mix) {
     if (p == nullptr) return fail(OCB_ERR_INVALID_ARG, "policy is NULL");
     if (p->generic) return fail(OCB_ERR_UNSUPPORTED, "the fused rollout kernel needs the tensor-core policy path (2 players, grids up to %d rows)", kMaxH);
     if (p->hidden != kHid) return fail(OCB_ERR_UNSUPPORTED, "the fused rollout kernel exists for hidden_size 64 only");
     if (population && tile_policy == nullptr) return fail(OCB_ERR_INVALID_ARG, "slice_policy is NULL");
     const bool cross = tile_policy != nullptr && !population;
+    const bool mixed = mix != nullptr;
+    if (mixed && (tile_policy != nullptr || population || values != nullptr || d_trace != nullptr))
+        return fail(OCB_ERR_INVALID_ARG, "mixed play takes no table, no critic and no trace");
     if (tile_policy == nullptr && (policy_index < 0 || policy_index >= p->n_policies)) return fail(OCB_ERR_INVALID_ARG, "policy index out of range");
+    if (mixed && (mix->partner_policy < 0 || mix->partner_policy >= p->n_policies))
+        return fail(OCB_ERR_INVALID_ARG, "policy index out of range");
     if (env_w != p->W || env_h != p->H) return fail(OCB_ERR_INVALID_ARG, "env and policy were built for different layouts");
     if (T < 1) return fail(OCB_ERR_INVALID_ARG, "T must be >= 1");
-    if (!cross && (obs_slab == nullptr || actions == nullptr || values == nullptr))
+    if (mixed && (mix->L < 2 || T != 2 * mix->L || envp.N % (mix->L - 1) != 0))
+        return fail(OCB_ERR_INVALID_ARG, "mixed play runs T = 2 L steps over a multiple of L - 1 worlds");
+    if (mixed && (obs_slab == nullptr || actions == nullptr)) return fail(OCB_ERR_INVALID_ARG, "obs_buf and actions are required");
+    if (!cross && !mixed && (obs_slab == nullptr || actions == nullptr || values == nullptr))
         return fail(OCB_ERR_INVALID_ARG, "obs_slab, actions and values are required");
     if (cross && (envp.N % kRows) != 0)
         return fail(OCB_ERR_INVALID_ARG, "cross-play needs a multiple of %d worlds (one weight set per 128-row tile of a seat), got %d", kRows, envp.N);
@@ -1743,6 +1767,10 @@ int ocb_policy_rollout_fused_launch(ocb_policy* p, int policy_index, const int32
     fp.env = envp;
     fp.T = T, fp.wtiles = wtiles, fp.slots = slots, fp.cross = cross ? 1 : 0;
     fp.obs_slab = obs_slab, fp.actions = actions, fp.logp = logp, fp.values = values, fp.reward = reward, fp.done = done;
+    if (mixed) {
+        fp.mix_L = mix->L, fp.mix_seed = mix->mix_seed, fp.mix_partner_seed = mix->partner_seed;
+        fp.mix_partner_blobs = p->d_blobs + (size_t)mix->partner_policy * 2 * (size_t)p->L.total;
+    }
     const int groups = (wtiles + slots - 1) / slots;
     const int ctas = groups < p->sm_count ? groups : p->sm_count;
     const size_t smem = (size_t)fused_smem_layout(p->npos, ring, p->S, p->SC, slots).total;
@@ -1757,11 +1785,17 @@ int ocb_policy_rollout_fused_launch(ocb_policy* p, int policy_index, const int32
         const int cols = 192 / (kCellCols * p->H);
         const char* e = getenv("OCB_FUSED_SPLIT");
         const bool want = e != nullptr ? (e[0] != '0') : true;
-        fp.col_ring = (want && slots == 1 && !cross && cols >= p->W) ? (p->W < kFMaxColRing ? p->W : kFMaxColRing) : 0;
+        fp.col_ring = (want && slots == 1 && !cross && !mixed && cols >= p->W) ? (p->W < kFMaxColRing ? p->W : kFMaxColRing) : 0;
         if (fp.col_ring < p->W) fp.col_ring = 0;
     }
     const cudaStream_t st = (cudaStream_t)stream;
-    if (population) {  // its own instances: the self-play and cross-play launches keep the code they had without this mode
+    if (mixed) {  // its own instances, like population: both actors are needed before the env step, so no split mode
+        fp.col_ring = kColRing;
+        if (slots == 2)
+            rollout_fused_kernel<false, false, 2, false, true><<<ctas, kFThreads, smem, st>>>(fp);
+        else
+            rollout_fused_kernel<false, false, 1, false, true><<<ctas, kFThreads, smem, st>>>(fp);
+    } else if (population) {  // its own instances: the self-play and cross-play launches keep the code they had without this mode
         if (fp.col_ring > 0) {
             rollout_fused_kernel<false, true, 1, true><<<ctas, kFThreads, smem, st>>>(fp);
         } else {

@@ -2,7 +2,8 @@
 // policy_kernels.cu inside its anonymous namespace, after the pair kernel whose roles it reuses).
 // Variants (FusedParams): one or two world tiles in flight per CTA (`slots`), split mode (the critic's conv stream deferred
 // behind the actor's; one tile in flight, whole grid resident in TMEM), cross-play (`cross`: two actors, seat-selected rows),
-// population self-play (`kPop`: the actor + critic of a weight set chosen per 128-world slice).
+// population self-play (`kPop`: the actor + critic of a weight set chosen per 128-world slice), mixed play (`kMix`: the
+// actors of two weight sets, a per-row draw picks which one acts, only the forced worlds are recorded).
 //
 // The 2T+1-launch rollout (ocb_rollout_policy) is bound by its dependent launches: per env step a
 // policy launch and an env launch, each of which fills and drains the GPU for one tile per SM.
@@ -48,6 +49,15 @@ struct FusedParams {
     // Population self-play (kernel instances with kPop, pol.f_seat1_tiles = 0) is not `cross`: the two networks are the
     // actor and critic of the slice's weight set and every row is emitted, as in self-play.
     int cross;
+    // Mixed play (kernel instances with kMix, T = 2 L, mixed_schedule.h): network 0 is the actor of the main weight set
+    // (pol.blobs), network 1 the actor at mix_partner_blobs.  Row r = seat N + n of world j = n mod (L - 1) plays main at step
+    // u if the world is forced (mix_forced_main) or the mask draw says so (!mix_draw_partner(mix_seed, r, step)), else the
+    // partner; epilogue group 0 emits the main rows (and the rows past N), group 1 the partner rows, the partner sampling
+    // with key mix_partner_seed.  Only forced worlds are recorded, at slot mix_record_slot of the [L, 2, N] buffers: group 0
+    // writes their actions and log-probs, the env warps their observation, reward and done.  No critic, nothing at u = T.
+    int mix_L;
+    unsigned long long mix_seed, mix_partner_seed;
+    const uint8_t* mix_partner_blobs;
 };
 
 constexpr int kFEnvWarps = 2;
@@ -222,13 +232,14 @@ struct FusedSlot {
     int cur_return, ep_add;
     long long ret_add;
     int n, nbytes;
+    int j;  // kMix: world index inside its replica (n mod (L - 1))
     bool valid, tma_ok, tma_pending;
     int8_t* obs_ptr;
     int32_t *rew_ptr, *done_ptr;
     uint32_t vts, acts;  // virtual tiles / action hand-offs of this slot so far (barrier phases); never reset
 };
 
-template <bool kProf, int kSlots>
+template <bool kProf, int kSlots, bool kMix = false>
 __device__ __forceinline__ void fused_env_role(const FusedParams& fp, uint8_t* s_env, const FusedSmemLayout& sl, const Tables& tb,
                                                const uint8_t* tmpl, const uint8_t* s_act, uint32_t bars) {
     constexpr int P = 2;
@@ -263,6 +274,10 @@ __device__ __forceinline__ void fused_env_role(const FusedParams& fp, uint8_t* s
                    ((reinterpret_cast<uintptr_t>(q.obs_ptr) & 15u) == 0) && ((obs_view_stride & 15u) == 0);
         q.rew_ptr = fp.reward ? fp.reward + q.n : nullptr;
         q.done_ptr = fp.done ? fp.done + q.n : nullptr;
+        if constexpr (kMix) {  // per-world stores of SC bytes: 16-byte aligned exactly when SC is
+            q.j = q.n % (fp.mix_L - 1);
+            q.tma_ok = store_obs && fp.env.use_tma && (SC & 15) == 0 && (reinterpret_cast<uintptr_t>(fp.obs_slab) & 15u) == 0;
+        }
         load_world<P, 1, 8>(tb, c, fp.env, nl, 0, objs_of(slot), q.w);
         q.cur_return = fp.env.cur_return[nl];
         q.ret_add = 0, q.ep_add = 0;
@@ -281,7 +296,9 @@ __device__ __forceinline__ void fused_env_role(const FusedParams& fp, uint8_t* s
         // finish long before the actions arrive, so these waits sit before the action wait, off the critical path)
         if (q.vts > 0) mbar_wait(bars + 8 * (FB_OBS_EMPTY + slot), (q.vts - 1) & 1);
         if (q.tma_pending) {
-            if (lane == 0) {
+            if (kMix) {
+                bulk_wait_read_all();  // every lane stores its own world's planes
+            } else if (lane == 0) {
                 if (other_pending)
                     bulk_wait_read_1();  // all but the newest group: the other slot's store may go on reading ITS planes
                 else
@@ -315,13 +332,21 @@ __device__ __forceinline__ void fused_env_role(const FusedParams& fp, uint8_t* s
                 reset_world<P>(tb, q.w);
                 for (int idx = 0; idx < c.n_objcells; ++idx) myobjs[(int)tb.objcells[idx] * 32] = 0;
             }
-            if (q.rew_ptr != nullptr) {
-                if (q.valid) q.rew_ptr[0] = r, q.rew_ptr[N] = r;
-                q.rew_ptr += PN;
-            }
-            if (q.done_ptr != nullptr) {
-                if (q.valid) *q.done_ptr = done ? 1 : 0;
-                q.done_ptr += N;
+            if constexpr (kMix) {  // the transition of step u - 1: recorded at the forced world's slot of that step
+                if (q.valid && mix_forced_main(fp.mix_L, u - 1, q.j)) {
+                    const size_t t = (size_t)mix_record_slot(fp.mix_L, u - 1, q.j);
+                    if (fp.reward != nullptr) fp.reward[t * PN + q.n] = r, fp.reward[t * PN + N + q.n] = r;
+                    if (fp.done != nullptr) fp.done[t * N + q.n] = done ? 1 : 0;
+                }
+            } else {
+                if (q.rew_ptr != nullptr) {
+                    if (q.valid) q.rew_ptr[0] = r, q.rew_ptr[N] = r;
+                    q.rew_ptr += PN;
+                }
+                if (q.done_ptr != nullptr) {
+                    if (q.valid) *q.done_ptr = done ? 1 : 0;
+                    q.done_ptr += N;
+                }
             }
             full = done;
             if (kProf && ew == 0) trace_ev<kProf>(fp.pol, (int)q.vts, 1);
@@ -333,7 +358,34 @@ __device__ __forceinline__ void fused_env_role(const FusedParams& fp, uint8_t* s
         mbar_arrive(bars + 8 * (FB_OBS_FULL + slot));  // release: the loaders may read this lane's planes
         if (kProf && ew == 0) trace_ev<kProf>(fp.pol, (int)q.vts, 3);
         ++q.vts;
-        if (store_obs) {
+        if (kMix && store_obs) {
+            // the observation a forced world acts on, at its slot of this step (u = T: no step, no record)
+            const bool rec = q.valid && u < T && mix_forced_main(fp.mix_L, u, q.j);
+            int8_t* dst = rec ? fp.obs_slab + ((size_t)mix_record_slot(fp.mix_L, u, q.j) * PN + q.n) * SC : nullptr;
+            if (q.tma_ok) {
+                if (rec) {
+                    fence_proxy_async_smem();
+#pragma unroll
+                    for (int v = 0; v < P; ++v)
+                        bulk_store_s2g(dst + v * obs_view_stride, smem_addr(myplanes) + v * view_stride, (uint32_t)SC);
+                    bulk_commit();
+                }
+                q.tma_pending = true;
+            } else {
+                // word copies, the warp on one world at a time (SC is a multiple of 4; rows are 4-byte aligned only)
+                __syncwarp();
+                for (uint32_t todo = __ballot_sync(0xFFFFFFFFu, rec); todo != 0u; todo &= todo - 1u) {
+                    const int b = __ffs(todo) - 1;
+                    int8_t* d = reinterpret_cast<int8_t*>(__shfl_sync(0xFFFFFFFFu, reinterpret_cast<unsigned long long>(dst), b));
+#pragma unroll
+                    for (int v = 0; v < P; ++v) {
+                        const uint32_t* s4 = reinterpret_cast<const uint32_t*>(planes + v * view_stride + b * SC);
+                        uint32_t* d4 = reinterpret_cast<uint32_t*>(d + v * obs_view_stride);
+                        for (int w4 = lane; w4 < (SC >> 2); w4 += 32) __stcs(d4 + w4, s4[w4]);
+                    }
+                }
+            }
+        } else if (store_obs) {
             int8_t* dst = q.obs_ptr + (size_t)u * obs_step_stride;
             if (q.tma_ok) {
                 fence_proxy_async_smem();
@@ -381,11 +433,13 @@ __device__ __forceinline__ void fused_env_role(const FusedParams& fp, uint8_t* s
         end_tile(sa, 0);
         if (kSlots == 2 && two) end_tile(sb, 1);
     }
-    if ((sa.tma_pending || (kSlots == 2 && sb.tma_pending)) && lane == 0) bulk_wait_read_all();
+    if ((sa.tma_pending || (kSlots == 2 && sb.tma_pending)) && (kMix || lane == 0)) bulk_wait_read_all();
 }
 
 // output stage of the epilogue in the fused rollout.  `net` = 0: six logits of the tile's rows, 1: head[0] = value.
 // Cross-play: both pipeline networks are actors; group 0 (net 0) owns the rows of seat 0, group 1 those of seat 1.
+// Mixed play (kMix): both are actors too; group 1 owns the rows the partner plays at this step, group 0 all others.
+template <bool kMix = false>
 struct FusedOut {
     const FusedParams& fp;
     uint8_t* s_act;
@@ -393,16 +447,38 @@ struct FusedOut {
     unsigned long long base;
     FusedCursor cur;
     int g;
+    bool partner_row;  // kMix: the partner plays this thread's row of the current virtual tile (set by draw)
     __device__ __forceinline__ FusedOut(const FusedParams& f, uint8_t* sa, uint32_t b) : fp(f), s_act(sa), bars(b), cur(f) {
         base = f.pol.offset;
         if (f.pol.d_offset != nullptr) base += *f.pol.d_offset;
         g = (int)(threadIdx.x >> 7);  // epilogue group of this thread
+        partner_row = false;
     }
-    __device__ __forceinline__ bool mine(int trow_id) const { return !fp.cross || (trow_id >> 6) == g; }
-    __device__ __forceinline__ uint32_t draw(int, int trow_id) const {
+    __device__ __forceinline__ bool mine(int trow_id) const {
+        if constexpr (kMix)
+            return partner_row == (g == 1);
+        else
+            return !fp.cross || (trow_id >> 6) == g;
+    }
+    // mixed_schedule.h, with the per-step path's counters (mask step = sampling offset = step counter + u); every row of the
+    // tile is claimed by exactly one group, or FB_ACT_FULL never completes: rows past N and the pass u = T go to group 0
+    __device__ __forceinline__ bool mix_partner_plays(int trow_id) const {
+        const int n = cur.kt() * kFWorlds + (trow_id & (kFWorlds - 1)), seat = trow_id >> 6;
+        if (n >= fp.env.N || cur.u >= fp.T || mix_forced_main(fp.mix_L, cur.u, n % (fp.mix_L - 1))) return false;
+        return mix_draw_partner(fp.mix_seed, (uint32_t)(seat * fp.env.N + n), base + (unsigned long long)cur.u);
+    }
+    __device__ __forceinline__ uint32_t draw(int, int trow_id) {
+        if constexpr (kMix) partner_row = mix_partner_plays(trow_id);
         if (fp.pol.deterministic || cur.u >= fp.T || !mine(trow_id)) return 0u;
         const int wl = trow_id & (kFWorlds - 1), seat = trow_id >> 6;
         const long long row = (long long)seat * fp.env.N + (cur.kt() * kFWorlds + wl);
+        if constexpr (kMix) {
+            if (g == 1) {  // the partner samples from its own stream: same counters, another key
+                PolicyParams kp = fp.pol;
+                kp.seed = fp.mix_partner_seed;
+                return policy_draw(kp, (uint32_t)row, base + (unsigned long long)cur.u);
+            }
+        }
         return policy_draw(fp.pol, (uint32_t)row, base + (unsigned long long)cur.u);
     }
     __device__ __forceinline__ void operator()(int, int trow_id, int net, const float (&head)[6], uint32_t drawn) {
@@ -415,15 +491,22 @@ struct FusedOut {
         } else if (u < fp.T && mine(trow_id)) {
             PolicyParams op = fp.pol;  // output pointers of this step; rows past N sample but store nothing
             const bool valid = n < N;
-            op.actions = valid ? fp.actions : nullptr, op.logp = valid ? fp.logp : nullptr, op.logits = nullptr;
-            emit_actor_row(op, store, (uint32_t)row, head, base + (unsigned long long)u, true, &drawn, s_act + cur.s * 128 + trow_id,
+            bool rec = valid;
+            long long at = store;
+            if constexpr (kMix) {  // a forced world's row (main's) lands at its slot; every other row stores nothing
+                const int j = valid ? n % (fp.mix_L - 1) : 0;
+                rec = valid && g == 0 && mix_forced_main(fp.mix_L, u, j);
+                at = ((long long)mix_record_slot(fp.mix_L, u, j) * 2 + seat) * N + n;
+            }
+            op.actions = rec ? fp.actions : nullptr, op.logp = rec ? fp.logp : nullptr, op.logits = nullptr;
+            emit_actor_row(op, at, (uint32_t)row, head, base + (unsigned long long)u, true, &drawn, s_act + cur.s * 128 + trow_id,
                            bars + 8 * (FB_ACT_FULL + cur.s));
         }
         cur.next();
     }
 };
 
-template <bool kProf, bool kSplit, int kSlots, bool kPop = false>
+template <bool kProf, bool kSplit, int kSlots, bool kPop = false, bool kMix = false>
 __global__ void __launch_bounds__(kFThreads, 1) rollout_fused_kernel(const FusedParams fp) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((128u - (smem_addr(smem_raw) & 127u)) & 127u);
@@ -481,7 +564,7 @@ __global__ void __launch_bounds__(kFThreads, 1) rollout_fused_kernel(const Fused
 
     long long pw[kProf ? PW_COUNT : 1] = {};
     if (warp < kEpiWarps) {
-        pair_epilogue_role<kProf, kSplit, kPop>(pw, prm, 0, nvt, L, tmem, s_head, bars, FusedOut(fp, s_act, bars));
+        pair_epilogue_role<kProf, kSplit, kPop, kMix>(pw, prm, 0, nvt, L, tmem, s_head, bars, FusedOut<kMix>(fp, s_act, bars));
     } else if (warp < kWarpMma) {
         fused_loader_role<kProf, kSplit>(fp, (uint32_t)nvt, tmem, s_env, sl, bars);
     } else if (warp == kWarpMma || warp == kWarpConv2) {
@@ -492,7 +575,8 @@ __global__ void __launch_bounds__(kFThreads, 1) rollout_fused_kernel(const Fused
         else
             pair_conv_role<kProf, -1>(pw, prm, 0, nvt, L, tmem, smem_addr(s_head), bars, half, 2);
     } else if (warp == kPWarpProd) {
-        pair_producer_role<kProf, kPop>(pw, prm, 0, nvt, L, smem_addr(s_head), smem_addr(s_wring), bars);
+        pair_producer_role<kProf, kPop, kMix>(pw, prm, 0, nvt, L, smem_addr(s_head), smem_addr(s_wring), bars,
+                                              kMix ? fp.mix_partner_blobs : nullptr);
     } else if (warp < kPWarpProd) {
         pair_fc_role<kProf, kSplit>(pw, prm, warp - kWarpFc, 0, nvt, L, tmem, smem_addr(s_wring), bars);
     } else if (warp == kFWarpConvC) {
@@ -500,7 +584,7 @@ __global__ void __launch_bounds__(kFThreads, 1) rollout_fused_kernel(const Fused
             pair_conv_role<kProf, 1>(pw, prm, 0, nvt, L, tmem, smem_addr(s_head), bars, 0, 1, (uint32_t)fp.col_ring, FB_COL_FULL,
                                      FB_COL_EMPTY);
     } else {
-        fused_env_role<kProf, kSlots>(fp, s_env, sl, *s_tables, s_tmpl, s_act, bars);
+        fused_env_role<kProf, kSlots, kMix>(fp, s_env, sl, *s_tables, s_tmpl, s_act, bars);
     }
     __syncwarp();
     tc_fence_before();

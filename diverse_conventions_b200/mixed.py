@@ -1,4 +1,5 @@
-"""Mixed-play ("MP") data collection on the device (``ocb_rollout_mixed``, csrc/mixed_kernels.cu).
+"""Mixed-play ("MP") data collection on the device (``ocb_rollout_mixed_fused``, csrc/rollout_fused.cuh, or the per-step
+``ocb_rollout_mixed``, csrc/mixed_kernels.cu).
 
 Replaces, for the CoMeDi / XD trainer of the reference:
 
@@ -10,15 +11,17 @@ Replaces, for the CoMeDi / XD trainer of the reference:
 * ``SharedReplayBuffer.diaginsert`` / ``partinsert`` (train/MAPPO/utils/shared_buffer.py:150-220): a dozen strided
   torch copies per step that put the forced worlds on a diagonal / a row prefix of the buffer.
 
-Here one env holds ``replicas`` independent copies of the G-world scheme, a collection is ``10 L + 4`` launches
-issued from C (or one CUDA-graph launch) and nothing synchronises.  The buffer is seat-major
+Here one env holds ``replicas`` independent copies of the G-world scheme and nothing synchronises.  A collection is one
+persistent launch of the fused rollout kernel plus one critic launch over the recorded observations (hidden 64, the layouts
+the tensor-core kernels take), else ``10 L + 4`` per-step launches; both issued from C (or one CUDA-graph launch), both
+filling the same buffers bit for bit.  The buffer is seat-major
 (``[L(+1), P, N, ...]``, int8 observations); ``shared_buffer_views()`` gives the reference's ``[L(+1), N, P, ...]``
 axis order as zero-copy views.
 """
 from __future__ import annotations
 
 import ctypes
-from typing import Dict
+from typing import Dict, Optional
 
 import torch
 
@@ -76,10 +79,15 @@ class MixedPlayCollector:
 
     ``policy`` holds the weight sets: ``main_policy`` = (actor being trained, its mixed-play critic ``mp_critic``,
     train/XD/MCPolicy.py:21,60), ``partner_policy`` = the partner convention (only its actor is used).  The env is
-    not reset: like the reference the collection continues from the env's current state."""
+    not reset: like the reference the collection continues from the env's current state.
+
+    ``fused``: ``None`` runs the collection as one persistent launch (``ocb_rollout_mixed_fused``) whenever it applies and
+    falls back to the per-step launches for good when the library answers ``OCB_ERR_UNSUPPORTED`` (hidden 512, layouts
+    outside the tensor-core kernels or too large for the fused kernel); ``True`` raises ``NativeError`` there instead;
+    ``False`` always runs the per-step path.  ``.fused`` tells which path ran."""
 
     def __init__(self, env: B200Overcooked, policy: FusedPolicy, L: int, main_policy: int = 0, partner_policy: int = 1,
-                 seed: int = 0, mix_seed: int = 0, use_graph: bool = False):
+                 seed: int = 0, mix_seed: int = 0, use_graph: bool = False, fused: Optional[bool] = None):
         if env.num_players != 2:
             raise ValueError("mixed play supports 2 players")
         if env.sim_device != policy.device:
@@ -97,17 +105,31 @@ class MixedPlayCollector:
         self.replicas = env.num_envs // (L - 1)
         self.buf = MixedPlayBuffer(env, L)
         self._lib = _native.lib()
-        nbytes = int(self._lib.ocb_rollout_mixed_scratch_bytes(env._h))
-        self._scratch = torch.empty((nbytes,), dtype=torch.uint8, device=env.sim_device)
+        self.fused = policy.hidden == 64 if fused is None else bool(fused)
+        self._fused_required = bool(fused)
+        self._scratch = None if fused else self._alloc_scratch()  # the per-step path's turn data, where that path can run
         self.use_graph = use_graph
         self._graph = None
         self.collections = 0
+
+    def _alloc_scratch(self) -> torch.Tensor:
+        nbytes = int(self._lib.ocb_rollout_mixed_scratch_bytes(self.env._h))
+        return torch.empty((nbytes,), dtype=torch.uint8, device=self.env.sim_device)
 
     def _issue(self, deterministic: bool):
         b, env = self.buf, self.env
         stream = ctypes.c_void_p(torch.cuda.current_stream(env.sim_device).cuda_stream)
         # launch-local sampling rows (a sharded PolicyRollout may have left global rows on a shared policy handle)
         _native.check(self._lib.ocb_policy_set_sampling_rows(self.policy._h, 0, 0, 0))
+        if self.fused:
+            rc = self._lib.ocb_rollout_mixed_fused(
+                env._h, self.policy._h, self.L, self.main_policy, self.partner_policy, _ptr(b.obs), _ptr(b.actions),
+                _ptr(b.action_log_probs), _ptr(b.value_preds), _ptr(b.rewards), _ptr(b.dones), int(deterministic),
+                self.seed, self.mix_seed, stream)
+            if rc != _native.OCB_ERR_UNSUPPORTED or self._fused_required:
+                _native.check(rc)
+                return
+            self.fused = False  # the library launched nothing: per-step launches from here on
         _native.check(self._lib.ocb_rollout_mixed(
             env._h, self.policy._h, self.L, self.main_policy, self.partner_policy, _ptr(b.obs), _ptr(b.actions),
             _ptr(b.action_log_probs), _ptr(b.value_preds), _ptr(b.rewards), _ptr(b.dones), int(deterministic), self.seed,

@@ -335,6 +335,19 @@ int ocb_rollout_mixed(ocb_env* env, ocb_policy* pol, int L, int main_policy, int
                       int32_t* actions, float* logp, float* values, int32_t* reward, int32_t* done, int deterministic,
                       uint64_t seed, uint64_t mix_seed, void* scratch, size_t scratch_bytes, void* stream);
 
+/* The same collection in ONE persistent launch of the fused rollout kernel (hidden 64): both actors run in the kernel's
+ * pipeline, the per-row switch, the forced worlds and their record at slot t happen on the device, then main_policy's critic
+ * runs once over the L * P * N rows of obs_buf[:L] (skipped when values == NULL) and slot L is written as above.  The same
+ * buffers, bit for bit, and the same final env state as ocb_rollout_mixed; buffer cells of rows that are not recorded are
+ * never written.  The env's step counter advances by 2L.  Needs no scratch; 5 launches with values, 3 without, on `stream`,
+ * no synchronisation, CUDA-graph capturable.  OCB_ERR_INVALID_ARG as ocb_rollout_mixed and for an obs_buf that is not
+ * 4-byte aligned (checked before anything is launched); OCB_ERR_UNSUPPORTED for hidden 512,
+ * for layouts outside the tensor-core kernels and for layouts too large for the fused kernel — callers then use
+ * ocb_rollout_mixed. */
+int ocb_rollout_mixed_fused(ocb_env* env, ocb_policy* pol, int L, int main_policy, int partner_policy, int8_t* obs_buf,
+                            int32_t* actions, float* logp, float* values, int32_t* reward, int32_t* done, int deterministic,
+                            uint64_t seed, uint64_t mix_seed, void* stream);
+
 /* ------------------------------------------------------- returns / GAE over the rollout buffer */
 /* SharedReplayBuffer.compute_returns (train/MAPPO/utils/shared_buffer.py:248-304) with the
  * ValueNorm de-normalisation (train/MAPPO/utils/valuenorm.py:76-87) and the advantage

@@ -7,14 +7,17 @@ or one rank per GPU under torchrun.
 
 selfplay : MAPPO self-play rollout (actor + critic forward of both seats, sampling, env step,
            PPO buffer write), random-init networks, hidden 64.
-mixed    : CoMeDi mixed-play collection (ocb_rollout_mixed): 2L env steps of replicas * (L-1) worlds, main policy
-           actor + critic and partner actor forward per step, per-row switch, diagonal / prefix buffer placement.
+mixed    : CoMeDi mixed-play collection: 2L env steps of replicas * (L-1) worlds, main and partner actor per step,
+           per-row switch, diagonal / prefix buffer placement, main critic on the recorded rows.  --fused 1: one
+           persistent launch + one value launch (ocb_rollout_mixed_fused), 0: 10L+4 per-step launches
+           (ocb_rollout_mixed), -1: auto, 2: both arms on identical envs, timed alternately --rounds times.
 crossplay: n x n pair matrix on coordination_ring, pairs sharded over the ranks, actors only,
            one 400-step episode per world, matrix gathered with one collective.
 Prints one JSON line per configuration (rank 0)."""
 import argparse
 import json
 import os
+import subprocess
 import sys
 
 import torch
@@ -44,6 +47,16 @@ def timed(fn, iters, world, dev):
     return float(ms.item()) / iters
 
 
+def power_limit(index):
+    """the card's power limit in W (nvidia-smi query), or None where it cannot be read"""
+    try:
+        out = subprocess.run(["nvidia-smi", "-i", str(index), "--query-gpu=power.limit", "--format=csv,noheader,nounits"],
+                             capture_output=True, text=True, timeout=30).stdout.strip()
+        return float(out)
+    except (OSError, ValueError, subprocess.SubprocessError):
+        return None
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--mode", default="selfplay", choices=["selfplay", "crossplay", "mixed"])
@@ -57,7 +70,9 @@ def main():
     ap.add_argument("--hidden", type=int, default=64, choices=[64, 512])
     ap.add_argument("--L", type=int, default=400, help="mixed: episode_length of the trainer")
     ap.add_argument("--replicas", type=int, default=20, help="mixed: copies of the (L-1)-world scheme per GPU")
-    ap.add_argument("--fused", type=int, default=-1, help="1: one persistent launch per rollout, 0: 2T+1 launches, -1: auto")
+    ap.add_argument("--fused", type=int, default=-1, help="1: one persistent launch per rollout, 0: 2T+1 launches, -1: auto"
+                    " (mixed: 2 = both arms, alternated)")
+    ap.add_argument("--rounds", type=int, default=5, help="mixed --fused 2: alternations of the two arms")
     args = ap.parse_args()
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -100,20 +115,52 @@ def main():
                 pol.set_weights(i, PolicyNet("actor", lp.width, lp.height, lp.channels, args.hidden).init_like_reference(1 + 100 * i),
                                 PolicyNet("critic", lp.width, lp.height, lp.channels, args.hidden).init_like_reference(2 + 100 * i))
             N = args.replicas * (args.L - 1)
-            env = B200Overcooked(layout, N, local, horizon=400, seed=1, world_offset=rank * N)
-            col = MixedPlayCollector(env, pol, args.L, 0, 1, seed=1, mix_seed=7 + rank, use_graph=bool(args.graph))
-            col.collect()
-            col.collect()
-            ms = timed(col.collect, args.iters, world, dev)
+            arms = [False, True] if args.fused == 2 else [None if args.fused < 0 else bool(args.fused)]
+            cols, envs = [], []
+            for fused in arms:
+                env = B200Overcooked(layout, N, local, horizon=400, seed=1, world_offset=rank * N)
+                col = MixedPlayCollector(env, pol, args.L, 0, 1, seed=1, mix_seed=7 + rank, use_graph=bool(args.graph),
+                                         fused=fused)
+                col.collect()
+                col.collect()
+                envs.append(env)
+                cols.append(col)
+            times = [[] for _ in cols]
+            for _ in range(args.rounds if args.fused == 2 else 1):
+                for i, col in enumerate(cols):
+                    times[i].append(timed(col.collect, args.iters, world, dev))
+            same = None
+            if len(cols) == 2:  # both arms ran the same collections from the same state: same buffers, bit for bit
+                torch.cuda.synchronize()
+                a, b = cols[0].buf, cols[1].buf
+                same = all(torch.equal(x, y) for x, y in zip(
+                    (a.obs, a.actions, a.action_log_probs, a.value_preds, a.rewards, a.dones),
+                    (b.obs, b.actions, b.action_log_probs, b.value_preds, b.rewards, b.dones)))
+            # the fused arm's critic pass on its own: main's critic (weight set 0) over the L * 2 * N recorded rows
+            value_ms = None
+            if any(col.fused for col in cols):
+                rows = cols[-1].buf.obs[:args.L]
+                vout = torch.empty((rows.numel() // (lp.width * lp.height * lp.channels),), dtype=torch.float32, device=dev)
+                pol.value(rows, out=vout)
+                value_ms = timed(lambda: pol.value(rows, out=vout), args.iters, world, dev)
             if rank == 0:
                 env_agent_steps = 2 * N * world * 2 * args.L
-                print(json.dumps({"mode": "mixed", "layout": layout, "hidden": args.hidden, "n_gpus": world, "L": args.L,
-                                  "replicas_per_gpu": args.replicas, "worlds_per_gpu": N, "graph": bool(args.graph),
-                                  "ms_per_collection": round(ms, 4), "us_per_env_step": round(1e3 * ms / (2 * args.L), 3),
-                                  "agent_steps_per_s": round(env_agent_steps / (ms * 1e-3)),
-                                  "recorded_agent_steps_per_s": round(env_agent_steps / 2 / (ms * 1e-3)),
-                                  "launches_per_collection": 10 * args.L + 4}), flush=True)
-            env.close()
+                for col, t in zip(cols, times):
+                    ms = sorted(t)[len(t) // 2]
+                    print(json.dumps({"mode": "mixed", "layout": layout, "hidden": args.hidden, "n_gpus": world, "L": args.L,
+                                      "replicas_per_gpu": args.replicas, "worlds_per_gpu": N, "world_tiles": (N + 63) // 64,
+                                      "graph": bool(args.graph), "fused": bool(col.fused),
+                                      "ms_per_collection": round(ms, 4), "ms_rounds": [round(x, 4) for x in t],
+                                      "us_per_env_step": round(1e3 * ms / (2 * args.L), 3),
+                                      "agent_steps_per_s": round(env_agent_steps / (ms * 1e-3)),
+                                      "recorded_agent_steps_per_s": round(env_agent_steps / 2 / (ms * 1e-3)),
+                                      # fused: rollout kernel, step-counter add, value pass, slot-L memset and fill
+                                      "launches_per_collection": 5 if col.fused else 10 * args.L + 4,
+                                      "ms_value_pass": round(value_ms, 4) if col.fused and value_ms is not None else None,
+                                      "arms_bit_identical": same, "gpu": torch.cuda.get_device_name(dev),
+                                      "power_limit_w": power_limit(local)}), flush=True)
+            for env in envs:
+                env.close()
             pol.close()
     else:
         layout = "random1"
