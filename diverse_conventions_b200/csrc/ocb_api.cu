@@ -709,6 +709,37 @@ extern "C" int ocb_rollout_crossplay_fused(ocb_env* e, ocb_policy* pol, int T, c
     return OCB_OK;
 }
 
+// Cross-play training rollout: the launch of ocb_rollout_crossplay_fused, unchanged, then one critic pass over obs_slab[0..T]
+// (ocb_policy_value_slab): the 128-row seat tiles with a critic_policy entry >= 0 get values[t] from that weight set's critic,
+// bit-identical to ocb_rollout_policy's; values of -1 tiles are never written.  Two launches, no scratch.
+extern "C" int ocb_rollout_crossplay_train_fused(ocb_env* e, ocb_policy* pol, int T, const int32_t* tile_policy,
+                                                 const int32_t* critic_policy, int8_t* obs_slab, int32_t* actions, float* logp,
+                                                 float* values, int32_t* reward, int32_t* done, int deterministic, uint64_t seed,
+                                                 void* stream) {
+    if (e == nullptr || pol == nullptr || tile_policy == nullptr || critic_policy == nullptr)
+        return fail(OCB_ERR_INVALID_ARG, "NULL handle / tile_policy / critic_policy");
+    if (obs_slab == nullptr || actions == nullptr || values == nullptr)
+        return fail(OCB_ERR_INVALID_ARG, "obs_slab, actions and values are required");
+    if (e->P != 2) return fail(OCB_ERR_UNSUPPORTED, "the policy rollout supports 2 players");
+    // what the critic pass would reject is rejected here, before the rollout launch
+    if ((reinterpret_cast<uintptr_t>(obs_slab) & 3u) != 0) return fail(OCB_ERR_INVALID_ARG, "obs_slab must be 4-byte aligned");
+    const long long rows = ((long long)T + 1) * 2 * e->N;
+    if (rows > kSlabMaxRows)
+        return fail(OCB_ERR_UNSUPPORTED, "the critic pass covers at most %d rows ((T + 1) * 2 N = %lld)", kSlabMaxRows, rows);
+    DeviceGuard guard(e->device);
+    RolloutParams p = base_params(e);
+    int rc = ocb_policy_rollout_fused_launch(pol, 0, tile_policy, false, p, e->h_tables.W, e->h_tables.H, T, obs_slab, actions, logp,
+                                             nullptr, reward, done, deterministic, seed,
+                                             reinterpret_cast<const uint64_t*>(e->d_step_counter),
+                                             reinterpret_cast<uint64_t*>(e->d_step_counter), stream);
+    if (rc != OCB_OK) return rc;
+    if (stream_capturing(stream))
+        e->count_stale = true;
+    else
+        e->step_count += (uint64_t)T;
+    return ocb_policy_value_slab(pol, obs_slab, T + 1, 2 * e->N / 128, critic_policy, values, stream);
+}
+
 // Self-play of a population in one persistent launch: the worlds [128 s, 128 s + 128) are played by weight set
 // slice_policy[s] on both seats, actor + critic — the buffers of ocb_rollout_policy(tile_policy = slice_policy ++
 // slice_policy, values != NULL), bit for bit.  Also writes obs_slab[0].

@@ -27,6 +27,15 @@ int ocb_policy_rollout_fused_launch(ocb_policy* pol, int policy_index, const int
 // ocb_policy_value with the critic of weight set `policy_index` and no table (hidden 64, tensor-core path only)
 int ocb_policy_value_of(ocb_policy* pol, int policy_index, const int8_t* obs, int M, float* values, void* stream);
 
+// Critic pass over a rollout slab obs_slab [steps][seat_tiles * 128 rows] (hidden 64, tensor-core path only): for every seat
+// tile k with critic_policy[k] >= 0 (DEVICE int32 [seat_tiles]) and every step t, values[t][k * 128 + r] = the critic of weight
+// set critic_policy[k] on row t * seat_tiles * 128 + k * 128 + r, bit-identical to ocb_policy_value; slots of tiles with -1 are
+// never written.  One launch of policy_pair_kernel's slab instance; the table is read on the device only (graph-capturable).
+// The row count steps * seat_tiles * 128 may not exceed kSlabMaxRows (OCB_ERR_UNSUPPORTED): the kernels index rows with int.
+constexpr int kSlabMaxRows = 0x7FFFFFFF;
+int ocb_policy_value_slab(ocb_policy* pol, const int8_t* obs_slab, int steps, int seat_tiles, const int32_t* critic_policy,
+                          float* values, void* stream);
+
 // bytes of one observation row the handle was built for (W * H * (5 P + 10)); 1 when shapes outside the tensor-core
 // kernels' range run through policy_generic_kernel
 int ocb_policy_obs_bytes(const ocb_policy* pol);

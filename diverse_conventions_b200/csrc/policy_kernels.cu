@@ -104,7 +104,7 @@ struct PolicyParams {
     size_t blob_stride;       // bytes between nets
     int W, H, S, SC, npos;
     const int8_t* obs;        // [M][SC]
-    int M, tiles;
+    int M, tiles;             // critic pass over a rollout slab (policy_pair_kernel<kProf, true>): tiles = seat tiles per step
     const int32_t* tile_policy;  // [tiles] or nullptr
     const int32_t* row_index;    // [M] source row of each forward row (obs / given_actions are indexed by it) or nullptr
     const int32_t* given_actions;  // evaluate_actions: log-prob of the stored action of the source row instead of sampling
@@ -131,6 +131,7 @@ struct PolicyParams {
     // tile_policy[kt / 2] / tile_policy[f_seat1_tiles + kt / 2] (the per-step path's seat-major 128-row tile table).
     // Population self-play (the kernel instances with kPop) sets f_seat1_tiles = 0 and a table by 128-world slice: fused_pair
     // gives p | p << 16 and the two networks are the actor and the critic of weight set p
+    // The critic pass over a rollout slab (policy_pair_kernel<kProf, true>) sets f_slots = the slab's steps (SlabWalk).
     int f_vt_round, f_slots, f_seat1_tiles;
 };
 
@@ -320,12 +321,38 @@ __device__ __forceinline__ bool blob_changed(const PolicyParams& prm, int t, int
     return prm.tile_policy[t] != prm.tile_policy[t - 1];
 }
 
+// critic pass over a rollout slab (policy_pair_kernel<kProf, true>, ocb_policy_value_slab): a unit is (seat tile k, step s)
+// for every seat tile whose table entry is >= 0, tile-major (all steps of tile k, then the next such tile), so a CTA's run of
+// units changes weights only where it crosses into a tile with another entry.  Each role walks the run with its own copy of
+// this cursor; unit (k, s) is the 128-row tile s * n + k of the slab (n = prm.tiles seat tiles per step, table
+// prm.tile_policy, prm.f_slots steps).
+struct SlabWalk {
+    int k, s, pol;  // the current unit and its weight set
+    __device__ __forceinline__ int tile(const PolicyParams& prm) const { return s * prm.tiles + k; }
+    // advance one unit; true when the new unit needs other weights than the previous one
+    __device__ __forceinline__ bool next(const PolicyParams& prm) {
+        if (++s < prm.f_slots) return false;
+        s = 0;
+        do ++k; while (k < prm.tiles && __ldg(prm.tile_policy + k) < 0);
+        const int np = k < prm.tiles ? __ldg(prm.tile_policy + k) : pol;  // the loader's look-ahead may step past the last unit
+        const bool chg = np != pol;
+        pol = np;
+        return chg;
+    }
+};
+// blob_changed of unit t of the run [t0, ...); the slab walk advances to unit t here
+template <bool kSlab>
+__device__ __forceinline__ bool unit_changed(const PolicyParams& prm, int t, int t0, SlabWalk& sw) {
+    if (!kSlab) return blob_changed(prm, t, t0);
+    return t == t0 || sw.next(prm);
+}
+
 // ---------------------------------------------------------------- roles
 // loader: global observations -> bf16 cell blocks, one grid column at a time; the two loader
 // groups take alternate columns of the CTA's column stream
-template <bool kProf>
+template <bool kProf, bool kSlab = false>
 __device__ __forceinline__ void loader_role(long long* pw, const PolicyParams& prm, const UnitRange ur, uint32_t tmem, uint32_t* s_stage,
-                                            uint32_t bars) {
+                                            uint32_t bars, SlabWalk sw = {}) {
     const int lwarp = (threadIdx.x >> 5) - kEpiWarps, lg = lwarp >> 2, lw = lwarp & 3, lane = threadIdx.x & 31;
     const int W = prm.W, H = prm.H, SC4 = prm.SC >> 2, seg = 5 * H, stride = prm.stage_stride;
     uint32_t* stg = s_stage + lwarp * 32 * stride;
@@ -340,8 +367,8 @@ __device__ __forceinline__ void loader_role(long long* pw, const PolicyParams& p
     int lt = ur.t0, lx = lg;
     while (lx >= W) lx -= W, ++lt;
     auto issue_loads = [&]() {
-        const long long r0 = (long long)lt * kRows + lw * 32;
-        if (prm.row_index != nullptr) {  // minibatch rows picked out of the rollout buffer (ocb_policy_evaluate)
+        const long long r0 = (long long)(kSlab ? sw.tile(prm) : lt) * kRows + lw * 32;
+        if (!kSlab && prm.row_index != nullptr) {  // minibatch rows picked out of the rollout buffer (ocb_policy_evaluate)
             long long mine = r0 + lane;
             mine = mine < prm.M ? mine : prm.M - 1;
             const int src = __ldg(prm.row_index + mine);
@@ -350,7 +377,7 @@ __device__ __forceinline__ void loader_role(long long* pw, const PolicyParams& p
                 const long long row = __shfl_sync(0xffffffffu, src, r);
                 pre[r] = active ? __ldg(obs32 + row * SC4 + lx * seg + lane) : 0u;
             }
-        } else if (r0 + 32 <= prm.M) {  // full 32-row slab: constant-stride addresses
+        } else if (kSlab || r0 + 32 <= prm.M) {  // full 32-row slab: constant-stride addresses (a rollout slab has only full tiles)
             const uint32_t* p = obs32 + r0 * SC4 + lx * seg + (active ? lane : 0);
 #pragma unroll
             for (int r = 0; r < 32; ++r) pre[r] = active ? __ldg(p + r * SC4) : 0u;
@@ -363,7 +390,10 @@ __device__ __forceinline__ void loader_role(long long* pw, const PolicyParams& p
             }
         }
         lx += 2;
-        while (lx >= W) lx -= W, ++lt;
+        while (lx >= W) {
+            lx -= W, ++lt;
+            if (kSlab) sw.next(prm);
+        }
     };
     if ((uint32_t)lg < ncols) issue_loads();
     for (uint32_t gc = lg; gc < ncols; gc += 2) {
@@ -568,10 +598,10 @@ __host__ __device__ inline PairSmemLayout pair_smem_layout(int npos, int ring, i
 
 // kPop (population self-play in the fused rollout): the two streams are the actor and critic of the slice's weight set
 // kMix (mixed play in the fused rollout): stream 0 is the actor at prm.blobs, stream 1 the actor at `mix_partner`
-template <bool kProf, bool kPop = false, bool kMix = false>
+template <bool kProf, bool kPop = false, bool kMix = false, bool kSlab = false>
 __device__ __forceinline__ void pair_producer_role(long long* pw, const PolicyParams& prm, int t0, int t1, const BlobLayout L,
                                                    uint32_t s_head, uint32_t s_wring, uint32_t bars,
-                                                   const uint8_t* mix_partner = nullptr) {
+                                                   const uint8_t* mix_partner = nullptr, SlabWalk sw = {}) {
     const int nets = prm.single ? 1 : 2;  // single mode: the one network takes the actor's places (stream 0, ring slots 0, 1, ...)
     const int R = prm.pair_ring, nch = nets * L.chunks;
     const bool resident = R >= nch;
@@ -582,8 +612,8 @@ __device__ __forceinline__ void pair_producer_role(long long* pw, const PolicyPa
     int slot = 0;
     for (int t = t0; t < t1; ++t, ++u) {
         if (static_w && u > 0) break;
-        const bool chg = blob_changed(prm, t, t0);
-        const int tp = tile_pol(prm, t);
+        const bool chg = unit_changed<kSlab>(prm, t, t0, sw);
+        const int tp = kSlab ? sw.pol : tile_pol(prm, t);
         const bool cross = prm.f_vt_round != 0 && prm.tile_policy != nullptr;  // both streams are actors (of two policies)
         const uint8_t* blob_a = prm.blobs + ((size_t)(cross ? (tp & 0xFFFF) : tp) * 2 + (prm.single == 2 ? 1 : 0)) * prm.blob_stride;
         const uint8_t* blob_c = kMix ? mix_partner
@@ -643,11 +673,11 @@ __device__ __forceinline__ void pair_producer_role(long long* pw, const PolicyPa
 // (position parity == accumulator stage), because ONE thread issuing 18 MMAs + commits + its waits per position
 // (~1.15 k cycles, tools/fused_trace.py) is slower than the epilogue that consumes them.  Every issuer releases a grid
 // column (col_empty) once none of ITS later positions reads it; the barrier counts the issuers.
-template <bool kProf, int kNet>
+template <bool kProf, int kNet, bool kSlab = false>
 __device__ __forceinline__ void pair_conv_role(long long* pw, const PolicyParams& prm, int t0, int t1, const BlobLayout L, uint32_t tmem,
                                                uint32_t a_head, uint32_t bars, const int cp0 = 0, const int cpstep = 1,
                                                const uint32_t ring = kColRing, const int col_full = PB_COL_FULL,
-                                               const int col_empty = PB_COL_EMPTY) {
+                                               const int col_empty = PB_COL_EMPTY, SlabWalk sw = {}) {
     const int W = prm.W, H = prm.H, PH = H - 2, npos = prm.npos;
     constexpr int kN = kNet < 0 ? kHid : kCo;
     const uint32_t idesc = make_idesc(kRows, kN);  // N = 64: actor channels 0-31 | critic channels 32-63
@@ -666,7 +696,7 @@ __device__ __forceinline__ void pair_conv_role(long long* pw, const PolicyParams
     };
 
     for (int t = t0; t < t1; ++t, ++u) {
-        if (blob_changed(prm, t, t0)) {
+        if (unit_changed<kSlab>(prm, t, t0, sw)) {
             mbar_wait_p<kProf>(bars + 8 * PB_HEAD_FULL, head_gen & 1, pw[PW_HEAD_FULL]);
             ++head_gen;
         }
@@ -911,9 +941,9 @@ constexpr int kSHeadGroup = 1;
 // every wait of this mode (211 us).  ncu: 47.7 k warp instructions per tile; the roles wait on each other in turn (role
 // profile, tools/policy_roles.py with OCB_PROFILE_MASK=1): loaders 60 % busy, conv issuers 60 %, epilogue groups 40 %.
 
-template <bool kProf>
+template <bool kProf, bool kSlab = false>
 __device__ __forceinline__ void single_fc_role(long long* pw, const PolicyParams& prm, int t0, int t1, const BlobLayout L, uint32_t tmem,
-                                               uint32_t a_wring, uint32_t bars) {
+                                               uint32_t a_wring, uint32_t bars, SlabWalk sw = {}) {
     const int npos = prm.npos;
     const int R = prm.pair_ring, nch = L.chunks;
     const bool resident = R >= nch;
@@ -924,7 +954,7 @@ __device__ __forceinline__ void single_fc_role(long long* pw, const PolicyParams
     uint32_t cnt0 = 0, cnt1 = 0;  // items consumed from group 0 / group 1
     int slot = 0;
     for (int t = t0; t < t1; ++t, ++u) {
-        const bool chg = blob_changed(prm, t, t0);
+        const bool chg = unit_changed<kSlab>(prm, t, t0, sw);
         const bool w_loaded = !resident || chg;
         if (resident && w_loaded) ++w_gen;
         for (int j = 0; j < npos + 2; ++j) {
@@ -961,12 +991,13 @@ __device__ __forceinline__ void single_fc_role(long long* pw, const PolicyParams
     }
 }
 
-template <bool kProf, class Out>
+template <bool kProf, bool kSlab = false, class Out>
 __device__ __forceinline__ void single_epilogue_role(long long* pw, const PolicyParams& prm, int t0, int t1, const BlobLayout L,
-                                                     uint32_t tmem, const uint8_t* s_head, uint32_t bars, Out&& out) {
+                                                     uint32_t tmem, const uint8_t* s_head, uint32_t bars, Out&& out,
+                                                     SlabWalk sw = {}) {
     const int warp = threadIdx.x >> 5, g = warp >> 2, trow_id = (warp & 3) * 32 + (threadIdx.x & 31);
     const int npos = prm.npos;
-    const int net = prm.single == 2 ? 1 : 0;  // head layout / outputs: 0 = actor (6 logits), 1 = critic (value)
+    const int net = (kSlab || prm.single == 2) ? 1 : 0;  // head layout / outputs: 0 = actor (6 logits), 1 = critic (value)
     const uint32_t trow = tmem + ((uint32_t)((warp & 3) * 32) << 16);
     const uint8_t* rest = s_head + kPRestOff - L.bias1;  // the network's bias1 .. bh at their blob offsets
     const float* s_bias1 = reinterpret_cast<const float*>(rest + L.bias1);
@@ -997,7 +1028,7 @@ __device__ __forceinline__ void single_epilogue_role(long long* pw, const Policy
         ++pubs;
     };
     for (int t = t0; t < t1; ++t, ++u) {
-        if (blob_changed(prm, t, t0)) {
+        if (unit_changed<kSlab>(prm, t, t0, sw)) {
             mbar_wait_p<kProf>(bars + 8 * PB_HEAD_FULL, head_gen & 1, pw[PW_HEAD_FULL]);
             ++head_gen;
         }
@@ -1038,7 +1069,7 @@ __device__ __forceinline__ void single_epilogue_role(long long* pw, const Policy
             head_accumulate(net, v, s_b2 + half * 32, s_wh, half * 32, head);
         }
         mbar_arrive(bars + 8 * (PB_HEAD_EMPTY + (u & 1)));
-        out(t, trow_id, net, head, drawn);
+        out(kSlab ? sw.tile(prm) : t, trow_id, net, head, drawn);
     }
 }
 
@@ -1065,7 +1096,46 @@ struct PairForwardOut {
     }
 };
 
-template <bool kProf>
+// kSlab: the critic over a rollout slab (single == 2): prm.tile_policy is the table of prm.tiles seat tiles per step,
+// prm.f_slots the number of steps and prm.M = steps * 128 * prm.tiles rows.  The CTA counts the tiles with an entry >= 0 (A) in the device table itself, takes its
+// even share [u0, u1) of the A * steps units and starts the walk at unit u0 (every thread scans a contiguous share of the
+// table; one block-wide prefix sum finds the tile of rank u0 / steps).
+__device__ __forceinline__ void slab_run(const PolicyParams& prm, uint32_t* s_scan, int* s_k0, SlabWalk& sw, int& u0, int& u1) {
+    const int n = prm.tiles, steps = prm.f_slots, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int per = (n + kPThreads - 1) / kPThreads, lo = tid * per < n ? tid * per : n, hi = lo + per < n ? lo + per : n;
+    int cnt = 0;
+    for (int i = lo; i < hi; ++i) cnt += __ldg(prm.tile_policy + i) >= 0;
+    int incl = cnt;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int v = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= d) incl += v;
+    }
+    if (lane == 31) s_scan[warp] = (uint32_t)incl;
+    __syncthreads();
+    int A = 0, excl = incl - cnt;
+    for (int w = 0; w < kPThreads / 32; ++w) {
+        A += (int)s_scan[w];
+        if (w < warp) excl += (int)s_scan[w];
+    }
+    const long long U = (long long)A * steps;
+    u0 = (int)(((long long)blockIdx.x * U) / gridDim.x);
+    u1 = (int)(((long long)(blockIdx.x + 1) * U) / gridDim.x);
+    const int r0 = u0 / steps;
+    if (u0 < u1 && r0 >= excl && r0 < excl + cnt) {  // this thread's share holds the run's first tile
+        int r = excl;
+        for (int i = lo; i < hi; ++i) {
+            if (__ldg(prm.tile_policy + i) < 0) continue;
+            if (r++ == r0) {
+                *s_k0 = i;
+                break;
+            }
+        }
+    }
+    sw.s = u0 - r0 * steps;
+}
+
+template <bool kProf, bool kSlab = false>
 __global__ void __launch_bounds__(kPThreads, 1) policy_pair_kernel(const PolicyParams prm) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((128u - (smem_addr(smem_raw) & 127u)) & 127u);
@@ -1099,6 +1169,11 @@ __global__ void __launch_bounds__(kPThreads, 1) policy_pair_kernel(const PolicyP
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
+    // the loaders' staging buffer is free until the roles start; the first tile of the slab run goes next to the TMEM slot
+    SlabWalk sw = {};
+    int* s_k0 = reinterpret_cast<int*>(s_bars + PB_TMEM_SLOT + 1);
+    int su0 = 0, su1 = 0;
+    if (kSlab) slab_run(prm, s_stage, s_k0, sw, su0, su1);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -1106,22 +1181,25 @@ __global__ void __launch_bounds__(kPThreads, 1) policy_pair_kernel(const PolicyP
     // tiles of this CTA
     UnitRange ur;
     ur.net = 0;
-    ur.t0 = (int)(((long long)blockIdx.x * prm.tiles) / gridDim.x);
-    ur.t1 = (int)(((long long)(blockIdx.x + 1) * prm.tiles) / gridDim.x);
+    ur.t0 = kSlab ? su0 : (int)(((long long)blockIdx.x * prm.tiles) / gridDim.x);
+    ur.t1 = kSlab ? su1 : (int)(((long long)(blockIdx.x + 1) * prm.tiles) / gridDim.x);
+    if (kSlab && su0 < su1) sw.k = *s_k0, sw.pol = __ldg(prm.tile_policy + sw.k);
 
     long long pw[kProf ? PW_COUNT : 1] = {};
     const long long t_begin = kProf ? clock64() : 0;
-    if (prm.single) {  // ONE network per tile (see single_epilogue_role)
+    if (kSlab || prm.single) {  // ONE network per tile (see single_epilogue_role)
         if (warp < kEpiWarps) {
-            single_epilogue_role<kProf>(pw, prm, ur.t0, ur.t1, L, tmem, s_head, bars, PairForwardOut(prm));
+            single_epilogue_role<kProf, kSlab>(pw, prm, ur.t0, ur.t1, L, tmem, s_head, bars, PairForwardOut(prm), sw);
         } else if (warp < kWarpMma) {
-            loader_role<kProf>(pw, prm, ur, tmem, s_stage, bars);
+            loader_role<kProf, kSlab>(pw, prm, ur, tmem, s_stage, bars, sw);
         } else if (warp == kWarpMma || warp == kWarpConv2) {
-            pair_conv_role<kProf, 0>(pw, prm, ur.t0, ur.t1, L, tmem, smem_addr(s_head), bars, warp == kWarpMma ? 0 : 1, 2);
+            pair_conv_role<kProf, 0, kSlab>(pw, prm, ur.t0, ur.t1, L, tmem, smem_addr(s_head), bars, warp == kWarpMma ? 0 : 1, 2,
+                                            kColRing, PB_COL_FULL, PB_COL_EMPTY, sw);
         } else if (warp == kPWarpProd) {
-            pair_producer_role<kProf>(pw, prm, ur.t0, ur.t1, L, smem_addr(s_head), smem_addr(s_wring), bars);
+            pair_producer_role<kProf, false, false, kSlab>(pw, prm, ur.t0, ur.t1, L, smem_addr(s_head), smem_addr(s_wring), bars,
+                                                           nullptr, sw);
         } else if (warp == kWarpFc) {
-            single_fc_role<kProf>(pw, prm, ur.t0, ur.t1, L, tmem, smem_addr(s_wring), bars);
+            single_fc_role<kProf, kSlab>(pw, prm, ur.t0, ur.t1, L, tmem, smem_addr(s_wring), bars, sw);
         }
     } else if (warp < kEpiWarps) {
         pair_epilogue_role<kProf, false>(pw, prm, ur.t0, ur.t1, L, tmem, s_head, bars, PairForwardOut(prm));
@@ -1307,6 +1385,7 @@ extern "C" int ocb_policy_create(const ocb_config* cfg, int device, int hidden, 
     const int smem_max = kSmemBudget + 128;
     if (err == cudaSuccess) err = cudaFuncSetAttribute(policy_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(policy_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(policy_pair_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<true, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(rollout_fused_kernel<false, true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
@@ -1667,6 +1746,33 @@ int ocb_policy_value_of(ocb_policy* p, int policy_index, const int8_t* obs, int 
     if (policy_index < 0 || policy_index >= p->n_policies) return fail(OCB_ERR_INVALID_ARG, "policy index out of range");
     return policy_launch(p, 2, obs, M, nullptr, nullptr, nullptr, nullptr, values, 0, 0, 0, nullptr, stream, nullptr, nullptr,
                          nullptr, policy_index);
+}
+
+int ocb_policy_value_slab(ocb_policy* p, const int8_t* obs_slab, int steps, int seat_tiles, const int32_t* critic_policy,
+                          float* values, void* stream) {
+    if (p == nullptr || obs_slab == nullptr || critic_policy == nullptr || values == nullptr)
+        return fail(OCB_ERR_INVALID_ARG, "NULL argument");
+    if (p->generic || p->hidden != kHid) return fail(OCB_ERR_UNSUPPORTED, "the slab critic pass exists for the hidden-64 tensor-core path");
+    if (steps < 1 || seat_tiles < 1) return fail(OCB_ERR_INVALID_ARG, "steps and seat_tiles must be >= 1");
+    if ((long long)steps * seat_tiles * kRows > kSlabMaxRows)
+        return fail(OCB_ERR_UNSUPPORTED, "the slab critic pass covers at most %d rows (got %d steps of %d rows)", kSlabMaxRows, steps,
+                    seat_tiles * kRows);
+    if ((reinterpret_cast<uintptr_t>(obs_slab) & 3u) != 0) return fail(OCB_ERR_INVALID_ARG, "obs_slab must be 4-byte aligned");
+    DeviceGuard guard(p->device);
+    PolicyParams prm;
+    memset(&prm, 0, sizeof(prm));
+    prm.blobs = p->d_blobs, prm.blob_stride = (size_t)p->L.total;
+    prm.W = p->W, prm.H = p->H, prm.S = p->S, prm.SC = p->SC, prm.npos = p->npos;
+    prm.obs = obs_slab, prm.M = steps * seat_tiles * kRows, prm.tiles = seat_tiles, prm.tile_policy = critic_policy;
+    prm.values = values, prm.f_slots = steps;
+    prm.net_mask = 2, prm.single = 2, prm.pair_ring = p->pair_ring, prm.stage_stride = p->stage_stride;
+    const long long units = (long long)steps * seat_tiles;  // an upper bound: the table is only read on the device
+    const int ctas = units < p->sm_count ? (int)units : p->sm_count;
+    policy_pair_kernel<false, true><<<ctas, kPThreads, p->pair_smem_bytes, (cudaStream_t)stream>>>(prm);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(OCB_ERR_CUDA, "slab critic pass launch failed: %s", cudaGetErrorString(err));
+    p->calls += 1;
+    return OCB_OK;
 }
 
 // Diagnostic: one fused forward with the instrumented build of the kernel.  h_prof (HOST, int64

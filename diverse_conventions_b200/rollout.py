@@ -131,7 +131,7 @@ class PolicyRollout:
     def __init__(self, env: B200Overcooked, policy: FusedPolicy, T: int, tile_policy: Optional[torch.Tensor] = None,
                  with_critic: bool = True, with_logp: bool = True, seed: int = 0, use_graph: bool = False,
                  fused: Optional[bool] = None, policy_index: int = 0, world_offset: int = 0,
-                 total_worlds: Optional[int] = None):
+                 total_worlds: Optional[int] = None, critic_policy: Optional[torch.Tensor] = None):
         """``total_worlds`` (with ``world_offset`` = global index of this env's world 0): key the action sampling by
         the GLOBAL (seat, world) so that a sharded run draws exactly the streams of the unsharded one
         (``ocb_policy_set_sampling_rows``); ``None`` keeps the launch-local rows.
@@ -142,7 +142,16 @@ class PolicyRollout:
         (``pair_tile_policy([(p0, p0), (p1, p1), ...], worlds_per_slice)``) with the critic on is population self-play:
         it runs as one launch too (``ocb_rollout_population_fused``).  The table is classified once, here: the launches
         read the caller's tensor, so in-place edits take effect (also in graph replays) but must keep the two halves
-        equal; build a new ``PolicyRollout`` for a table that mixes policies across seats."""
+        equal; build a new ``PolicyRollout`` for a table that mixes policies across seats.
+
+        ``critic_policy`` (int32 ``[2N/128]``, the seat tiles of ``tile_policy``; needs ``tile_policy`` and ``with_critic``):
+        cross-play TRAINING collection, XD's SP / XP slices.  Seat tile k acts with ``tile_policy[k]``'s actor and is valued
+        by ``critic_policy[k]``'s critic, or not at all for -1 (a partner's seat): its ``value_preds`` slots stay 0.0.
+        ``crossplay_training_tables`` builds both tables.  ``fused=None`` runs the cross-play launch plus one critic pass
+        (``ocb_rollout_crossplay_train_fused``), falling back to per-step actor launches and per-step critic passes where
+        that is unsupported (hidden 512, layouts outside the fused kernel); ``fused=True`` raises ``NativeError`` there.
+        Both tables are checked once, here (entries -1 or below ``n_policies``; ``tile_policy`` entries 0 or more); the
+        launches read the caller's tensors."""
         if env.num_players != policy.layout.num_players:
             raise ValueError("env and policy were built for different player counts")
         if env.sim_device != policy.device:
@@ -154,8 +163,20 @@ class PolicyRollout:
             if tile_policy.dtype != torch.int32 or tile_policy.numel() != (M + TILE - 1) // TILE:
                 raise ValueError("tile_policy must be int32 [%d]" % ((M + TILE - 1) // TILE))
             tile_policy = tile_policy.to(env.sim_device).contiguous()
+        if critic_policy is not None:
+            if tile_policy is None or not with_critic:
+                raise ValueError("critic_policy needs tile_policy and with_critic=True")
+            if env.num_envs % TILE != 0:
+                raise ValueError("critic_policy needs a multiple of %d worlds (one critic per 128-row seat tile)" % TILE)
+            if critic_policy.dtype != torch.int32 or critic_policy.numel() != tile_policy.numel():
+                raise ValueError("critic_policy must be int32 [%d]" % tile_policy.numel())
+            critic_policy = critic_policy.to(env.sim_device).contiguous()
+            for name, table, low in (("tile_policy", tile_policy, 0), ("critic_policy", critic_policy, -1)):
+                host = table.cpu()
+                if bool(((host < low) | (host >= policy.n_policies)).any()):
+                    raise ValueError("%s entries must lie in [%d, %d)" % (name, low, policy.n_policies))
         self.env, self.policy, self.T, self.seed = env, policy, T, seed
-        self.tile_policy = tile_policy
+        self.tile_policy, self.critic_policy = tile_policy, critic_policy
         self.buf = RolloutBuffer(env, T, with_critic, with_logp)
         self._lib = _native.lib()
         self.policy_index = policy_index
@@ -165,7 +186,14 @@ class PolicyRollout:
         # or self-play slices of a population with their critics: ocb_rollout_population_fused)
         small = policy.hidden == 64 and env.num_players == 2
         self._slice_policy = None
-        if tile_policy is not None and with_critic and env.num_players == 2 and env.num_envs % TILE == 0:
+        if critic_policy is not None:
+            # slots of -1 tiles are never written by the fused path; the per-step fallback zeroes them after its critic pass
+            self.buf.value_preds.zero_()
+            self._no_value = (critic_policy < 0).view(1, -1, 1)
+            self._critic_filled = critic_policy.clamp(min=0)  # -1 -> weight set 0, whose values are then zeroed
+            self.fused = small if fused is None else bool(fused)
+            self._fused_required = bool(fused)
+        elif tile_policy is not None and with_critic and env.num_players == 2 and env.num_envs % TILE == 0:
             half = tile_policy.numel() // 2
             host = tile_policy.cpu()
             if torch.equal(host[:half], host[half:]):
@@ -177,11 +205,13 @@ class PolicyRollout:
             raise _native.NativeError(_native.OCB_ERR_UNSUPPORTED, "the population launch exists for hidden_size 64 only")
         # fused=True on a population table of a layout the fused kernel does not take (generic-kernel layouts, layouts too
         # large for its shared memory) is answered by the launch itself: OCB_ERR_UNSUPPORTED, raised at collect()
-        if fused and not (can_fuse or population):
+        # (so is fused=True with a critic_policy: hidden 512 included)
+        if fused and not (can_fuse or population or critic_policy is not None):
             raise ValueError("the fused rollout needs hidden 64, two players and either self-play of one policy with its critic "
                              "or cross-play slices (tile_policy, a multiple of %d worlds) without one" % TILE)
-        self.fused = can_fuse if fused is None else bool(fused)
-        self._fused_required = bool(fused)
+        if critic_policy is None:
+            self.fused = can_fuse if fused is None else bool(fused)
+            self._fused_required = bool(fused)
         if tile_policy is None and policy_index != 0 and not self.fused:
             self.tile_policy = tile_policy = torch.full(((M + TILE - 1) // TILE,), policy_index, dtype=torch.int32,
                                                         device=env.sim_device)
@@ -201,7 +231,12 @@ class PolicyRollout:
         # handle-level state, set per issue: several rollouts may share one policy handle
         _native.check(self._lib.ocb_policy_set_sampling_rows(self.policy._h, *self._sampling_rows))
         if self.fused:
-            if self._slice_policy is not None:
+            if self.critic_policy is not None:
+                rc = self._lib.ocb_rollout_crossplay_train_fused(
+                    env._h, self.policy._h, self.T, _ptr(self.tile_policy), _ptr(self.critic_policy), _ptr(b.obs),
+                    _ptr(b.actions), _ptr(b.action_log_probs), _ptr(b.value_preds), _ptr(b.rewards), _ptr(b.dones),
+                    int(deterministic), self.seed, stream)
+            elif self._slice_policy is not None:
                 rc = self._lib.ocb_rollout_population_fused(
                     env._h, self.policy._h, self.T, _ptr(self._slice_policy), _ptr(b.obs), _ptr(b.actions),
                     _ptr(b.action_log_probs), _ptr(b.value_preds), _ptr(b.rewards), _ptr(b.dones), int(deterministic),
@@ -218,10 +253,26 @@ class PolicyRollout:
                 _native.check(rc)
                 return
             self.fused = False  # layout too large for the fused kernel: per-step launches from here on
+        if self.critic_policy is not None:
+            self._issue_crossplay_train_steps(deterministic, stream)
+            return
         _native.check(self._lib.ocb_rollout_policy(
             env._h, self.policy._h, self.T, _ptr(self.tile_policy), _ptr(b.obs), _ptr(b.actions),
             _ptr(b.action_log_probs), _ptr(b.value_preds), _ptr(b.rewards), _ptr(b.dones), int(deterministic),
             self.seed, stream))
+
+    def _issue_crossplay_train_steps(self, deterministic: bool, stream):
+        """the per-step form of ocb_rollout_crossplay_train_fused: the actors through ocb_rollout_policy without a critic, then
+        one critic pass per step (a single pass over all T + 1 steps would size the hidden-512 activation scratch for the
+        whole slab), then the slots of -1 tiles zeroed"""
+        b, env, M = self.buf, self.env, self.env.num_players * self.env.num_envs
+        _native.check(self._lib.ocb_rollout_policy(
+            env._h, self.policy._h, self.T, _ptr(self.tile_policy), _ptr(b.obs), _ptr(b.actions), _ptr(b.action_log_probs),
+            None, _ptr(b.rewards), _ptr(b.dones), int(deterministic), self.seed, stream))
+        for t in range(self.T + 1):
+            _native.check(self._lib.ocb_policy_value(self.policy._h, _ptr(b.obs[t]), M, _ptr(self._critic_filled),
+                                                     _ptr(b.value_preds[t]), stream))
+        b.value_preds.view(self.T + 1, -1, TILE).masked_fill_(self._no_value, 0.0)
 
     def prime(self):
         """slot 0 <- observation of the env's CURRENT state.  Always re-observed (one cheap launch): the env may have
@@ -280,6 +331,22 @@ class PolicyRollout:
 
 
 # ---------------------------------------------------------------------------- cross-play
+def crossplay_training_tables(slices: Sequence, worlds_per_slice: int, device=None):
+    """(tile_policy, critic_policy) of a cross-play training collection (``PolicyRollout(..., critic_policy=...)``): the env's
+    worlds are ``len(slices)`` contiguous slices of ``worlds_per_slice`` worlds, slice s given as ``((actor0, critic0),
+    (actor1, critic1))`` weight-set indices per seat; a critic of ``None`` (a seat whose values are not needed) becomes -1.
+
+    XD (train/XD/xd_player.py:177-230), the ego ``e`` with SP / XP critics ``sp``, ``xp0[j]``, ``xp1[j]`` against partners
+    ``p[j]``: ``[((e, sp), (e, sp))] + [((e, xp0[j]), (p[j], None)) for j] + [((p[j], None), (e, xp1[j])) for j]``.  Best
+    response (train/MultiConvention/xd_player.py:66-171): ``[((e, e), (p[j], None)) for j] + [((p[j], None), (e, e)) for j]``."""
+    sl = [tuple(tuple(seat) for seat in s) for s in slices]
+    if not sl or any(len(s) != 2 or any(len(seat) != 2 for seat in s) for s in sl):
+        raise ValueError("each slice is ((actor0, critic0), (actor1, critic1))")
+    actors = pair_tile_policy([(s[0][0], s[1][0]) for s in sl], worlds_per_slice, device)
+    critics = pair_tile_policy([tuple(-1 if seat[1] is None else seat[1] for seat in s) for s in sl], worlds_per_slice, device)
+    return actors, critics
+
+
 def pair_tile_policy(pairs: Sequence[Sequence[int]], worlds_per_pair: int, device=None) -> torch.Tensor:
     """tile_policy of an env whose worlds are ``len(pairs)`` contiguous slices of ``worlds_per_pair``
     worlds, slice s played by (seat 0: policy pairs[s][0], seat 1: policy pairs[s][1]) — the layout of

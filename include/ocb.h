@@ -289,6 +289,23 @@ int ocb_rollout_crossplay_fused(ocb_env* env, ocb_policy* pol, int T, const int3
                                 int32_t* actions, float* logp, int32_t* reward, int32_t* done, int deterministic,
                                 uint64_t seed, void* stream);
 
+/* Cross-play TRAINING rollout (the SP / XP collection of XDPlayer, train/XD/xd_player.py:177-230, and MultiConvention's
+ * best-response collection, train/MultiConvention/xd_player.py:66-171): the launch of ocb_rollout_crossplay_fused with
+ * `tile_policy`, then ONE critic pass over obs_slab[0..T] (the bootstrap slot T included).  `critic_policy` (DEVICE int32
+ * [2 N / 128], the seat-major tiles of tile_policy) names the weight set whose critic values each 128-row seat tile, or -1 for
+ * a tile that needs no values (a partner's seat; its weight set may have no critic).  values [T+1, 2, N]: slots of tiles with
+ * an entry >= 0 get the values ocb_rollout_policy would write with that critic, bit for bit; slots of -1 tiles are never
+ * written.  Table entries are not checked (they stay on the device; an entry >= n_policies reads outside the weights).
+ * obs_slab, actions, values and both tables are required; logp, reward, done may be NULL.  The errors of
+ * ocb_rollout_crossplay_fused (OCB_ERR_UNSUPPORTED for hidden 512 and for layouts outside the fused kernel; OCB_ERR_INVALID_ARG
+ * when N is not a multiple of 128), OCB_ERR_INVALID_ARG for an obs_slab that is not 4-byte aligned and OCB_ERR_UNSUPPORTED for
+ * a slab of more than 2^31 - 1 rows ((T + 1) * 2 N) are all reported before anything is launched.  Two launches on `stream`,
+ * no scratch, no synchronisation, CUDA-graph capturable; the env's step counter advances by T. */
+int ocb_rollout_crossplay_train_fused(ocb_env* env, ocb_policy* pol, int T, const int32_t* tile_policy,
+                                      const int32_t* critic_policy, int8_t* obs_slab, int32_t* actions, float* logp,
+                                      float* values, int32_t* reward, int32_t* done, int deterministic, uint64_t seed,
+                                      void* stream);
+
 /* Self-play of a population in ONE persistent launch (the per-member self-play slices of ADAP's simultaneous trainer and of
  * XD's conventions, train/ADAP/simultaneous.py, train/XD/serial.py): the worlds [128 s, 128 s + 128) are played by weight
  * set slice_policy[s] on both seats, actor + critic, hidden 64.  slice_policy: DEVICE int32 [N / 128], every entry in
