@@ -25,6 +25,14 @@ _u64 = ctypes.c_uint64
 _sz = ctypes.c_size_t
 _pp = ctypes.POINTER(ctypes.c_void_p)
 
+
+
+class ocb_weight_src(ctypes.Structure):
+    """one network of ``ocb_policy_set_weights_device``: (policy, net) and eight DEVICE fp32 pointers"""
+    _fields_ = [("policy", ctypes.c_int), ("net", ctypes.c_int)] + [
+        (name, ctypes.c_void_p) for name in ("conv_w", "conv_b", "fc1_w", "fc1_b", "fc2_w", "fc2_b", "head_w", "head_b")]
+
+
 # name -> (restype, argtypes); must list every function declared in include/ocb.h
 PROTOTYPES = {
     "ocb_abi_version": (_i, []),
@@ -57,6 +65,8 @@ PROTOTYPES = {
     "ocb_policy_create": (_i, [ctypes.POINTER(ocb_config), _i, _i, _i, _pp]),
     "ocb_policy_destroy": (_i, [_vp]),
     "ocb_policy_set_weights": (_i, [_vp, _i, _i] + [_vp] * 8),
+    "ocb_policy_set_weights_device": (_i, [_vp, _i, _vp, _vp]),
+    "ocb_policy_read_blob": (_i, [_vp, _i, _i, _vp, _sz, _vp]),
     "ocb_policy_act": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _u64, _u64, _vp]),
     "ocb_policy_act_ex": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _u64, _u64, _vp, _vp]),
     "ocb_policy_value": (_i, [_vp, _vp, _i, _vp, _vp, _vp]),

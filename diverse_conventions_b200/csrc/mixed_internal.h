@@ -32,7 +32,8 @@ struct MixRecordParams {
 
 cudaError_t launch_mix_select(const MixSelectParams& p, cudaStream_t stream);
 cudaError_t launch_mix_record(const MixRecordParams& p, cudaStream_t stream);
-cudaError_t launch_fill_f32(float* a, size_t n, float v, cudaStream_t stream);
+// a[0 .. n) = *v, read when the kernel runs (v is a DEVICE address)
+cudaError_t launch_fill_f32(float* a, size_t n, const float* v, cudaStream_t stream);
 cudaError_t launch_fill2_i32(int32_t* a, int n0, int v0, int32_t* b, int n1, int v1, cudaStream_t stream);
 
 }  // namespace ocb

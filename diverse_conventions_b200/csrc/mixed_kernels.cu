@@ -69,14 +69,14 @@ __global__ void fill_i32_kernel(int32_t* a, int n0, int v0, int32_t* b, int n1, 
     if (i < n1) b[i] = v1;
 }
 
-__global__ void fill_f32_kernel(float* a, size_t n, float v) {
+__global__ void fill_f32_kernel(float* a, size_t n, const float* v) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) a[i] = v;
+    if (i < n) a[i] = *v;
 }
 
 }  // namespace
 
-cudaError_t launch_fill_f32(float* a, size_t n, float v, cudaStream_t stream) {
+cudaError_t launch_fill_f32(float* a, size_t n, const float* v, cudaStream_t stream) {
     if (n == 0) return cudaSuccess;
     fill_f32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(a, n, v);
     return cudaGetLastError();

@@ -903,9 +903,10 @@ extern "C" int ocb_rollout_mixed(ocb_env* e, ocb_policy* pol, int L, int main_po
     // slot L is never written by the collection (diaginsert / partinsert stop at L-1): the reference bootstraps from
     // the all-zero observation the buffer was created with (MainPlayer.compute_one on mp_buf.share_obs[-1]); the
     // critic's value of it is a constant of the weights (the tensor-core forward folds the terrain planes of real
-    // observations into its bias, so it is evaluated on the host when the weights are set)
+    // observations into its bias, so it is evaluated when the weights are set) and is read where it lives on the device, so
+    // a replayed graph fills the value of the critic loaded at replay time
     OCB_CU(cudaMemsetAsync(obs_buf + (size_t)L * obs_step, 0, obs_step, st));
-    if (values != nullptr) OCB_CU(launch_fill_f32(values + (size_t)L * PN, PN, ocb_policy_zero_obs_value(pol, main_policy), st));
+    if (values != nullptr) OCB_CU(launch_fill_f32(values + (size_t)L * PN, PN, ocb_policy_zero_value_device(pol, main_policy), st));
     return OCB_OK;
 #undef OCB_CU
 }
@@ -950,7 +951,7 @@ extern "C" int ocb_rollout_mixed_fused(ocb_env* e, ocb_policy* pol, int L, int m
     }
     cudaError_t err = cudaMemsetAsync(obs_buf + (size_t)L * obs_step, 0, obs_step, st);
     if (err == cudaSuccess && values != nullptr)
-        err = launch_fill_f32(values + (size_t)L * PN, PN, ocb_policy_zero_obs_value(pol, main_policy), st);
+        err = launch_fill_f32(values + (size_t)L * PN, PN, ocb_policy_zero_value_device(pol, main_policy), st);
     if (err != cudaSuccess) {
         cudaGetLastError();
         return fail(OCB_ERR_CUDA, "ocb_rollout_mixed_fused: %s", cudaGetErrorString(err));

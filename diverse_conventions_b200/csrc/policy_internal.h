@@ -42,5 +42,6 @@ int ocb_policy_obs_bytes(const ocb_policy* pol);
 int ocb_policy_is_generic(const ocb_policy* pol);
 // number of (actor, critic) weight sets the handle holds
 int ocb_policy_num_sets(const ocb_policy* pol);
-// R_Critic value of the all-zero observation under weight set `policy` (computed on the host at set_weights)
-float ocb_policy_zero_obs_value(const ocb_policy* pol, int policy);
+// DEVICE address of the R_Critic value of the all-zero observation under weight set `policy` (written by both set_weights
+// paths when they pack the critic; 0 before that), nullptr for a bad index
+const float* ocb_policy_zero_value_device(const ocb_policy* pol, int policy);

@@ -416,7 +416,7 @@ __device__ __forceinline__ void loader_role(long long* pw, const PolicyParams& p
             uint32_t w[5];
 #pragma unroll
             for (int q = 0; q < 5; ++q) w[q] = mine[y * 5 + q];
-            // chunk 0: channels 0..7 ; chunk 1: channels 8, 9, 16, 17, 18, 19, 15, pad (slot_channel[] on the host)
+            // chunk 0: channels 0..7 ; chunk 1: channels 8, 9, 16, 17, 18, 19, 15, pad (slot_channel())
             const uint4 c0 = make_uint4(bytes_bf16x2(w[0], pair_sel(0, 1)), bytes_bf16x2(w[0], pair_sel(2, 3)),
                                         bytes_bf16x2(w[1], pair_sel(0, 1)), bytes_bf16x2(w[1], pair_sel(2, 3)));
             const uint4 c1 = make_uint4(bytes_bf16x2(w[2], pair_sel(0, 1)), bytes_bf16x2(w[4], pair_sel(0, 1)),
@@ -1230,26 +1230,259 @@ __global__ void __launch_bounds__(kPThreads, 1) policy_pair_kernel(const PolicyP
 #include "rollout_fused.cuh"
 #include "policy_generic.cuh"
 
-// ---------------------------------------------------------------- host-side packing
-uint16_t bf16_bits(float x) {
+// ---------------------------------------------------------------- packing rules
+// One definition for both writers of a blob: ocb_policy_set_weights (host loops over HOST weights) and policy_pack_kernel
+// (ocb_policy_set_weights_device, DEVICE weights).  Both must produce the same bytes, so every rounding here is explicit.
+__host__ __device__ inline uint16_t bf16_bits(float x) {
     uint32_t u;
     memcpy(&u, &x, 4);
     const uint32_t r = u + 0x7FFFu + ((u >> 16) & 1u);  // round to nearest even
     return (uint16_t)(r >> 16);
 }
-float bf16_val(uint16_t b) {
+__host__ __device__ inline float bf16_val(uint16_t b) {
     uint32_t u = (uint32_t)b << 16;
     float f;
     memcpy(&f, &u, 4);
     return f;
 }
 // element (n, k) of an [N x K] K-major operand in the canonical no-swizzle layout
-size_t canon_off(int n, int k, int K) { return (size_t)(n / 8) * (K / 8) * 128 + (size_t)(k / 8) * 128 + (n % 8) * 16 + (k % 8) * 2; }
-void put_split(uint8_t* hi, uint8_t* lo, size_t off, float w) {
+__host__ __device__ inline size_t canon_off(int n, int k, int K) {
+    return (size_t)(n / 8) * (K / 8) * 128 + (size_t)(k / 8) * 128 + (n % 8) * 16 + (k % 8) * 2;
+}
+__host__ __device__ inline void put_split(uint8_t* hi, uint8_t* lo, size_t off, float w) {
     const uint16_t h = bf16_bits(w);
     const uint16_t l = bf16_bits(w - bf16_val(h));
     memcpy(hi + off, &h, 2);
     memcpy(lo + off, &l, 2);
+}
+// observation channel of bf16 slot s of a cell block (== loader_role): channels 0-9, 16-19, 15, one zero pad (-1)
+__host__ __device__ inline int slot_channel(int s) { return s < 10 ? s : s < 14 ? s + 6 : s == 14 ? 15 : -1; }
+// element (co, k = window cell j * kSlots + slot) of the conv operand [co x 144]; conv_w is [CO, 20, 3, 3]
+__host__ __device__ inline float conv_slot_weight(const float* conv_w, int co, int k) {
+    const int j = k / kSlots, ch = slot_channel(k % kSlots);
+    return ch < 0 ? 0.0f : conv_w[((co * 20 + ch) * 3 + j / 3) * 3 + j % 3];
+}
+// conv bias of output position pos plus the static terrain channels (shift+0..4 == channels 10..14, one-hot of terrain-1;
+// setup_base_observation, envs/overcooked2_reimplement.py:165-171), summed in double in this order and rounded once
+__host__ __device__ inline float terrain_bias(const uint8_t* terrain, int W, int H, const float* conv_w, const float* conv_b,
+                                              int pos, int co) {
+    const int PH = H - 2, ox = pos / PH, oy = pos % PH;
+    double acc = conv_b[co];
+    for (int dx = 0; dx < 3; ++dx)
+        for (int dy = 0; dy < 3; ++dy) {
+            const int t = terrain[(oy + dy) * W + ox + dx];
+            if (t >= 1 && t <= 5) acc += conv_w[((co * 20 + 10 + (t - 1)) * 3 + dx) * 3 + dy];
+        }
+    return (float)acc;
+}
+
+// R_Critic.forward on an all-zero observation: the conv output is its bias at every position (flatten index co*npos + pos,
+// cnn.py:41), then FC -> ReLU -> FC -> ReLU -> v_out.  Each unit is a sequential sum in k with every product and every sum
+// rounded on its own: the device spells that out (nvcc would contract them into FMAs), the host build (-O3 for plain x86-64)
+// has no FMA instruction to contract into.
+__host__ __device__ inline float mul_rn(float a, float b) {
+#ifdef __CUDA_ARCH__
+    return __fmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+__host__ __device__ inline float add_rn(float a, float b) {
+#ifdef __CUDA_ARCH__
+    return __fadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+// unit o of the first hidden layer, after the ReLU
+__host__ __device__ inline float zero_obs_fc1(int o, int hidden, int npos, const float* conv_b, const float* fc1_w,
+                                              const float* fc1_b) {
+    const int co_n = hidden / 2;
+    const float* w = fc1_w + (size_t)o * co_n * npos;
+    float acc = fc1_b[o];
+    for (int co = 0; co < co_n; ++co) {
+        const float x = fmaxf(conv_b[co], 0.0f);
+        for (int pos = 0; pos < npos; ++pos) acc = add_rn(acc, mul_rn(w[co * npos + pos], x));
+    }
+    return fmaxf(acc, 0.0f);
+}
+// b + w . x over n inputs (FC2 units and the value head)
+__host__ __device__ inline float zero_obs_dot(float b, const float* w, const float* x, int n) {
+    float acc = b;
+    for (int k = 0; k < n; ++k) acc = add_rn(acc, mul_rn(w[k], x[k]));
+    return acc;
+}
+
+// ---------------------------------------------------------------- device-side packing (ocb_policy_set_weights_device)
+// One launch packs up to kPackMax networks: blockIdx.y = network, the last block of every row computes the zero-observation
+// value of a critic, the others walk the blob in 16-byte units.  A unit inside a bf16 hi operand packs one canonical core-matrix
+// row (8 K-consecutive elements) into hi AND lo; units inside lo operands are skipped; every other unit is fp32 (padding as
+// zeros), so every byte of the blob is written and the result does not depend on what was there.
+constexpr int kPackMax = 40;       // descriptors per launch (a 4 KB kernel-parameter block)
+constexpr int kPackThreads = 256;
+constexpr int kPackMaxBlocks = 1024;
+enum : int { PACK_H64 = 0, PACK_H512 = 1, PACK_GENERIC = 2 };
+
+struct PackDesc {
+    uint8_t* dst;  // the blob
+    const float *conv_w, *conv_b, *fc1_w, *fc1_b, *fc2_w, *fc2_b, *head_w, *head_b;
+    int policy, net;
+};
+struct PackArgs {
+    int fmt, W, H, C, npos, hidden, n;
+    size_t blob_bytes;
+    const uint8_t* terrain;  // [W * H] terrain codes of the layout
+    float* zero_value;       // [n_policies]
+    PackDesc d[kPackMax];
+};
+
+// row `row` of an [N x K] operand (rows enumerated in canonical order, so consecutive threads store consecutive 16 bytes);
+// wf(n, k) gives the fp32 weight
+template <class WF>
+__device__ __forceinline__ void pack_split_row(uint8_t* hi, uint8_t* lo, int row, int K, WF wf) {
+    const int n = (row / K) * 8 + row % 8, k0 = (row / 8) % (K / 8) * 8;
+    uint4 h, l;
+#pragma unroll
+    for (int kk = 0; kk < 8; ++kk) put_split(reinterpret_cast<uint8_t*>(&h), reinterpret_cast<uint8_t*>(&l), kk * 2, wf(n, k0 + kk));
+    const size_t o = canon_off(n, k0, K);
+    *reinterpret_cast<uint4*>(hi + o) = h;
+    *reinterpret_cast<uint4*>(lo + o) = l;
+}
+
+// the fp32 word at byte offset o of a hidden-64 blob's head (bias1 .. bh)
+__device__ float pack_f32_h64(const PackArgs& a, const PackDesc& d, const BlobLayout& L, int o) {
+    if (o < L.b1) {
+        const int i = (o - L.bias1) / 4;
+        return i < a.npos * kCo ? terrain_bias(a.terrain, a.W, a.H, d.conv_w, d.conv_b, i / kCo, i % kCo) : 0.0f;
+    }
+    if (o < L.b2) return d.fc1_b[(o - L.b1) / 4];
+    if (o < L.wh) return d.fc2_b[(o - L.b2) / 4];
+    if (o < L.bh) {
+        const int i = (o - L.wh) / 4;
+        if (d.net == 0) return i % 8 < 6 ? d.head_w[(i % 8) * kHid + i / 8] : 0.0f;  // hidden-major [64][8]
+        return i < kHid ? d.head_w[i] : 0.0f;
+    }
+    const int i = (o - L.bh) / 4;
+    return i < (d.net == 0 ? 6 : 1) ? d.head_b[i] : 0.0f;
+}
+
+// the fp32 word at byte offset o of a Blob5 outside its bf16 operands
+__device__ float pack_f32_h512(const PackArgs& a, const PackDesc& d, const Blob5& L, size_t o) {
+    const int head_out = d.net == 0 ? 6 : 1;
+    if (o < L.w1) {
+        const int i = (int)((o - L.bias1) / 4);
+        return terrain_bias(a.terrain, a.W, a.H, d.conv_w, d.conv_b, i / kCo5, i % kCo5);
+    }
+    if (o < L.w2) return d.fc1_b[(o - L.b1) / 4];
+    if (o < L.wh) return d.fc2_b[(o - L.b2) / 4];
+    if (o < L.bh) {
+        const size_t i = (o - L.wh) / 4;
+        return i < (size_t)head_out * kH5 ? d.head_w[i] : 0.0f;
+    }
+    const size_t i = (o - L.bh) / 4;
+    return i < (size_t)head_out ? d.head_b[i] : 0.0f;
+}
+
+// float i of a GBlob (the transposes of ocb_policy_set_weights' generic branch)
+__device__ float pack_f32_generic(const PackArgs& a, const PackDesc& d, const GBlob& G, size_t i) {
+    const int C = a.C, h = a.hidden, CO = h / 2, np = a.npos, head_out = d.net == 0 ? 6 : 1;
+    if (i < G.conv_b) {
+        const size_t x = i - G.conv_w;
+        const int co = (int)(x % CO), c = (int)(x / CO % C), ij = (int)(x / CO / C);
+        return d.conv_w[((size_t)(co * C + c) * 3 + ij / 3) * 3 + ij % 3];
+    }
+    if (i < G.w1) return d.conv_b[i - G.conv_b];
+    if (i < G.b1) {
+        const size_t x = i - G.w1;
+        const int n = (int)(x % h), co = (int)(x / h % CO), pos = (int)(x / h / CO);
+        return d.fc1_w[(size_t)n * (CO * np) + (size_t)co * np + pos];
+    }
+    if (i < G.w2) return d.fc1_b[i - G.b1];
+    if (i < G.b2) {
+        const size_t x = i - G.w2;
+        return d.fc2_w[(x % h) * h + x / h];
+    }
+    if (i < G.wh) return d.fc2_b[i - G.b2];
+    if (i < G.bh) {
+        const size_t x = i - G.wh;
+        return x / h < (size_t)head_out ? d.head_w[x] : 0.0f;
+    }
+    return i - G.bh < (size_t)head_out ? d.head_b[i - G.bh] : 0.0f;
+}
+
+// the zero-observation value of critic d (one block): zero_obs_fc1 / zero_obs_dot with the units spread over the threads
+__device__ void pack_zero_value(const PackArgs& a, const PackDesc& d) {
+    __shared__ float x1[kH5], x2[kH5];
+    const int h = a.hidden;
+    for (int o = threadIdx.x; o < h; o += blockDim.x) x1[o] = zero_obs_fc1(o, h, a.npos, d.conv_b, d.fc1_w, d.fc1_b);
+    __syncthreads();
+    for (int o = threadIdx.x; o < h; o += blockDim.x) x2[o] = fmaxf(zero_obs_dot(d.fc2_b[o], d.fc2_w + (size_t)o * h, x1, h), 0.0f);
+    __syncthreads();
+    if (threadIdx.x == 0) a.zero_value[d.policy] = zero_obs_dot(d.head_b[0], d.head_w, x2, h);
+}
+
+__global__ void __launch_bounds__(kPackThreads) policy_pack_kernel(const __grid_constant__ PackArgs a) {
+    const PackDesc& d = a.d[blockIdx.y];
+    if (blockIdx.x == gridDim.x - 1) {
+        if (d.net == 1) pack_zero_value(a, d);
+        return;
+    }
+    uint8_t* const b = d.dst;
+    const int npos = a.npos;
+    const size_t units = a.blob_bytes / 16, stride = (size_t)(gridDim.x - 1) * blockDim.x;
+    for (size_t u = (size_t)blockIdx.x * blockDim.x + threadIdx.x; u < units; u += stride) {
+        const size_t o = u * 16;
+        float f[4];
+        if (a.fmt == PACK_H64) {
+            const BlobLayout L = blob_layout(npos);
+            const int oi = (int)o;
+            if (oi < L.wc_lo) {
+                pack_split_row(b + L.wc_hi, b + L.wc_lo, oi / 16, kK1, [&](int n, int k) { return conv_slot_weight(d.conv_w, n, k); });
+                continue;
+            }
+            if (oi < L.bias1) continue;
+            if (oi >= L.head_bytes) {  // FC chunk c: [64 x 32] hi | lo; chunks npos, npos + 1 = the K halves of W2
+                const int c = (oi - L.head_bytes) / kChunk, r = (oi - L.head_bytes) % kChunk;
+                if (r >= kChunk / 2) continue;
+                uint8_t* hi = b + L.head_bytes + (size_t)c * kChunk;
+                if (c < npos)
+                    pack_split_row(hi, hi + kChunk / 2, r / 16, kCo,
+                                   [&](int n, int k) { return d.fc1_w[(size_t)n * (kCo * npos) + k * npos + c]; });
+                else
+                    pack_split_row(hi, hi + kChunk / 2, r / 16, 32,
+                                   [&](int n, int k) { return d.fc2_w[n * kHid + (c - npos) * 32 + k]; });
+                continue;
+            }
+            for (int j = 0; j < 4; ++j) f[j] = pack_f32_h64(a, d, L, oi + 4 * j);
+        } else if (a.fmt == PACK_H512) {
+            const Blob5 L = blob5_layout(npos);
+            if (o < L.wc_lo) {
+                pack_split_row(b + L.wc_hi, b + L.wc_lo, (int)(o / 16), kK1, [&](int n, int k) { return conv_slot_weight(d.conv_w, n, k); });
+                continue;
+            }
+            if (o < L.bias1) continue;
+            const bool in_w1 = o >= L.w1 && o < L.b1, in_w2 = o >= L.w2 && o < L.b2;
+            if (in_w1 || in_w2) {  // K block kc: [512 x 16] hi | lo
+                const size_t base = in_w1 ? L.w1 : L.w2;
+                const int kc = (int)((o - base) / kWBlk), r = (int)((o - base) % kWBlk);
+                if (r >= kWBlk / 2) continue;
+                uint8_t* hi = b + base + (size_t)kc * kWBlk;
+                if (in_w1)  // packed K index k = pos * 256 + co
+                    pack_split_row(hi, hi + kWBlk / 2, r / 16, kKc, [&](int n, int k) {
+                        const int kg = kc * kKc + k;
+                        return d.fc1_w[(size_t)n * (kCo5 * npos) + (size_t)(kg % kCo5) * npos + kg / kCo5];
+                    });
+                else
+                    pack_split_row(hi, hi + kWBlk / 2, r / 16, kKc, [&](int n, int k) { return d.fc2_w[(size_t)n * kH5 + kc * kKc + k]; });
+                continue;
+            }
+            for (int j = 0; j < 4; ++j) f[j] = pack_f32_h512(a, d, L, o + 4 * j);
+        } else {
+            const GBlob G = gblob_layout(a.C, a.hidden, npos);
+            for (int j = 0; j < 4; ++j) f[j] = pack_f32_generic(a, d, G, u * 4 + j);
+        }
+        *reinterpret_cast<float4*>(b + o) = make_float4(f[0], f[1], f[2], f[3]);
+    }
 }
 
 }  // namespace
@@ -1269,9 +1502,11 @@ struct ocb_policy {
     Blob5 L5;
     uint8_t* d_scratch;
     size_t scratch_tiles;
-    // critic value of the all-zero observation per weight set (a constant of the weights; the mixed-play buffer
-    // bootstraps from the never-written slot L, which holds zeros in the reference)
-    std::vector<float> zero_value;
+    // critic value of the all-zero observation per weight set, on the device (a constant of the weights, written by
+    // whichever path packs the critic; the mixed-play buffer bootstraps from the never-written slot L, which holds zeros in
+    // the reference, and reads it when the launch runs, so a replayed graph sees the current critic)
+    float* d_zero_value = nullptr;
+    uint8_t* d_terrain = nullptr;  // [S] terrain codes, for the device-side fold of the static planes
     uint32_t rng_rows_per_seat = 0, rng_add0 = 0, rng_add1 = 0;  // ocb_policy_set_sampling_rows
     // generic mode (policy_generic.cuh): shapes outside the tensor-core kernels' range (P != 2, H > 6, one conv position)
     int generic = 0;
@@ -1286,6 +1521,8 @@ extern "C" int ocb_policy_destroy(ocb_policy* p) {
     cudaFree(p->d_scratch);
     cudaFree(p->d_blobs);
     cudaFree(p->d_gblobs);
+    cudaFree(p->d_zero_value);
+    cudaFree(p->d_terrain);
     delete p;
     return OCB_OK;
 }
@@ -1293,29 +1530,17 @@ extern "C" int ocb_policy_destroy(ocb_policy* p) {
 int ocb_policy_num_sets(const ocb_policy* p) { return p ? p->n_policies : 0; }
 int ocb_policy_obs_bytes(const ocb_policy* p) { return p ? p->SC : 0; }
 int ocb_policy_is_generic(const ocb_policy* p) { return p ? p->generic : 0; }
-float ocb_policy_zero_obs_value(const ocb_policy* p, int policy) {
-    return (p && policy >= 0 && policy < (int)p->zero_value.size()) ? p->zero_value[policy] : 0.0f;
+const float* ocb_policy_zero_value_device(const ocb_policy* p, int policy) {
+    return (p && policy >= 0 && policy < p->n_policies) ? p->d_zero_value + policy : nullptr;
 }
 
-// R_Critic.forward on an all-zero observation, fp32 on the host: the conv output is its bias at every position
-// (flatten index co*npos + pos, cnn.py:41), then FC -> ReLU -> FC -> ReLU -> v_out
+// the zero-observation critic value on the host (the rules of pack_zero_value, one unit after the other)
 static float zero_obs_value(int hidden, int npos, const float* conv_b, const float* fc1_w, const float* fc1_b,
                             const float* fc2_w, const float* fc2_b, const float* head_w, const float* head_b) {
-    const int co_n = hidden / 2, k1 = co_n * npos;
     std::vector<float> x1((size_t)hidden), x2((size_t)hidden);
-    for (int o = 0; o < hidden; ++o) {
-        float acc = fc1_b[o];
-        for (int k = 0; k < k1; ++k) acc += fc1_w[(size_t)o * k1 + k] * fmaxf(conv_b[k / npos], 0.0f);
-        x1[o] = fmaxf(acc, 0.0f);
-    }
-    for (int o = 0; o < hidden; ++o) {
-        float acc = fc2_b[o];
-        for (int k = 0; k < hidden; ++k) acc += fc2_w[(size_t)o * hidden + k] * x1[k];
-        x2[o] = fmaxf(acc, 0.0f);
-    }
-    float v = head_b[0];
-    for (int k = 0; k < hidden; ++k) v += head_w[k] * x2[k];
-    return v;
+    for (int o = 0; o < hidden; ++o) x1[o] = zero_obs_fc1(o, hidden, npos, conv_b, fc1_w, fc1_b);
+    for (int o = 0; o < hidden; ++o) x2[o] = fmaxf(zero_obs_dot(fc2_b[o], fc2_w + (size_t)o * hidden, x1.data(), hidden), 0.0f);
+    return zero_obs_dot(head_b[0], head_w, x2.data(), hidden);
 }
 
 extern "C" int ocb_policy_create(const ocb_config* cfg, int device, int hidden, int n_policies, ocb_policy** out) {
@@ -1374,6 +1599,10 @@ extern "C" int ocb_policy_create(const ocb_config* cfg, int device, int hidden, 
     cudaError_t err = cudaDeviceGetAttribute(&p->sm_count, cudaDevAttrMultiProcessorCount, device);
     if (err == cudaSuccess) err = cudaMalloc(&p->d_blobs, bytes);
     if (err == cudaSuccess) err = cudaMemset(p->d_blobs, 0, bytes);
+    if (err == cudaSuccess) err = cudaMalloc(&p->d_zero_value, (size_t)n_policies * sizeof(float));
+    if (err == cudaSuccess) err = cudaMemset(p->d_zero_value, 0, (size_t)n_policies * sizeof(float));
+    if (err == cudaSuccess) err = cudaMalloc(&p->d_terrain, (size_t)p->S);
+    if (err == cudaSuccess) err = cudaMemcpy(p->d_terrain, p->terrain.data(), (size_t)p->S, cudaMemcpyHostToDevice);
     if (generic) {
         const size_t gbytes = (size_t)n_policies * 2 * p->LG.total * sizeof(float);
         if (err == cudaSuccess) err = cudaMalloc(&p->d_gblobs, gbytes);
@@ -1415,28 +1644,14 @@ static int set_weights512(ocb_policy* p, int policy, int net, const float* conv_
                           const float* fc1_b, const float* fc2_w, const float* fc2_b, const float* head_w, const float* head_b) {
     const Blob5& L = p->L5;
     std::vector<uint8_t> blob(L.total, 0);
-    const int npos = p->npos, PH = p->H - 2;
-    static const int slot_channel[kSlots] = {0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 16, 17, 18, 19, 15, -1};  // == loader_role
+    const int npos = p->npos;
     for (int co = 0; co < kCo5; ++co)
-        for (int j = 0; j < 9; ++j)
-            for (int s = 0; s < kSlots; ++s) {
-                const int ch = slot_channel[s];
-                const float w = ch < 0 ? 0.0f : conv_w[((co * 20 + ch) * 3 + j / 3) * 3 + j % 3];
-                put_split(blob.data() + L.wc_hi, blob.data() + L.wc_lo, canon_off(co, j * kSlots + s, kK1), w);
-            }
+        for (int k = 0; k < kK1; ++k)
+            put_split(blob.data() + L.wc_hi, blob.data() + L.wc_lo, canon_off(co, k, kK1), conv_slot_weight(conv_w, co, k));
     float* bias1 = reinterpret_cast<float*>(blob.data() + L.bias1);
-    for (int pos = 0; pos < npos; ++pos) {
-        const int ox = pos / PH, oy = pos % PH;
-        for (int co = 0; co < kCo5; ++co) {
-            double acc = conv_b[co];
-            for (int dx = 0; dx < 3; ++dx)
-                for (int dy = 0; dy < 3; ++dy) {
-                    const int t = p->terrain[(oy + dy) * p->W + ox + dx];
-                    if (t >= 1 && t <= 5) acc += conv_w[((co * 20 + 10 + (t - 1)) * 3 + dx) * 3 + dy];
-                }
-            bias1[pos * kCo5 + co] = (float)acc;
-        }
-    }
+    for (int pos = 0; pos < npos; ++pos)
+        for (int co = 0; co < kCo5; ++co)
+            bias1[pos * kCo5 + co] = terrain_bias(p->terrain.data(), p->W, p->H, conv_w, conv_b, pos, co);
     // FC1: packed K index k = pos * 256 + co; block kc holds k in [32 kc, 32 kc + 32)
     const int K1 = kCo5 * npos;
     for (int n = 0; n < kH5; ++n) {
@@ -1532,8 +1747,13 @@ extern "C" int ocb_policy_set_weights(ocb_policy* p, int policy, int net, const 
         return fail(OCB_ERR_INVALID_ARG, "NULL argument");
     if (policy < 0 || policy >= p->n_policies || net < 0 || net > 1) return fail(OCB_ERR_INVALID_ARG, "bad policy / net index");
     if (net == 1) {
-        p->zero_value.resize((size_t)p->n_policies, 0.0f);
-        p->zero_value[policy] = zero_obs_value(p->hidden, p->npos, conv_b, fc1_w, fc1_b, fc2_w, fc2_b, head_w, head_b);
+        const float v = zero_obs_value(p->hidden, p->npos, conv_b, fc1_w, fc1_b, fc2_w, fc2_b, head_w, head_b);
+        DeviceGuard guard(p->device);
+        const cudaError_t err = cudaMemcpy(p->d_zero_value + policy, &v, sizeof(float), cudaMemcpyHostToDevice);
+        if (err != cudaSuccess) {
+            cudaGetLastError();
+            return fail(OCB_ERR_CUDA, "ocb_policy_set_weights: %s", cudaGetErrorString(err));
+        }
     }
     if (p->generic) {  // fp32, transposed so that consecutive output units are consecutive words (policy_generic.cuh)
         const GBlob& G = p->LG;
@@ -1569,31 +1789,14 @@ extern "C" int ocb_policy_set_weights(ocb_policy* p, int policy, int net, const 
     if (p->hidden == kH5) return set_weights512(p, policy, net, conv_w, conv_b, fc1_w, fc1_b, fc2_w, fc2_b, head_w, head_b);
     const BlobLayout& L = p->L;
     std::vector<uint8_t> blob((size_t)L.total, 0);
-    const int npos = p->npos, H = p->H, PH = H - 2;
-    static const int slot_channel[kSlots] = {0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 16, 17, 18, 19, 15, -1};  // == loader_role
+    const int npos = p->npos;
     for (int co = 0; co < kCo; ++co)
-        for (int j = 0; j < 9; ++j)
-            for (int s = 0; s < kSlots; ++s) {
-                const int ch = slot_channel[s];
-                const float w = ch < 0 ? 0.0f : conv_w[((co * 20 + ch) * 3 + j / 3) * 3 + j % 3];
-                put_split(blob.data() + L.wc_hi, blob.data() + L.wc_lo, canon_off(co, j * kSlots + s, kK1), w);
-            }
-    // static terrain channels (shift+0..4 == channels 10..14, one-hot of terrain-1; setup_base_observation,
-    // envs/overcooked2_reimplement.py:165-171) folded into a per-position bias
+        for (int k = 0; k < kK1; ++k)
+            put_split(blob.data() + L.wc_hi, blob.data() + L.wc_lo, canon_off(co, k, kK1), conv_slot_weight(conv_w, co, k));
+    // the static terrain planes folded into a per-position bias
     float* bias1 = reinterpret_cast<float*>(blob.data() + L.bias1);
-    for (int pos = 0; pos < npos; ++pos) {
-        const int ox = pos / PH, oy = pos % PH;
-        for (int co = 0; co < kCo; ++co) {
-            double acc = conv_b[co];
-            for (int dx = 0; dx < 3; ++dx)
-                for (int dy = 0; dy < 3; ++dy) {
-                    const int x = ox + dx, y = oy + dy;
-                    const int t = p->terrain[y * p->W + x];
-                    if (t >= 1 && t <= 5) acc += conv_w[((co * 20 + 10 + (t - 1)) * 3 + dx) * 3 + dy];
-                }
-            bias1[pos * kCo + co] = (float)acc;
-        }
-    }
+    for (int pos = 0; pos < npos; ++pos)
+        for (int co = 0; co < kCo; ++co) bias1[pos * kCo + co] = terrain_bias(p->terrain.data(), p->W, p->H, conv_w, conv_b, pos, co);
     // FC chunks: chunk pos = W1 of that position [64 x 32]; chunks npos, npos+1 = the K halves of W2 [64 x 32]
     uint8_t* chunks = blob.data() + L.head_bytes;
     for (int n = 0; n < kHid; ++n) {
@@ -1625,6 +1828,97 @@ extern "C" int ocb_policy_set_weights(ocb_policy* p, int policy, int net, const 
         return fail(OCB_ERR_CUDA, "ocb_policy_set_weights: %s", cudaGetErrorString(err));
     }
     return OCB_OK;
+}
+
+// blob of (policy, net) and its size in bytes, in whichever of the three formats the handle uses
+static uint8_t* blob_of(const ocb_policy* p, int policy, int net, size_t* bytes) {
+    const size_t unit = (size_t)policy * 2 + net;
+    if (p->generic) {
+        *bytes = p->LG.total * sizeof(float);
+        return reinterpret_cast<uint8_t*>(p->d_gblobs + unit * p->LG.total);
+    }
+    *bytes = p->hidden == kH5 ? p->L5.total : (size_t)p->L.total;
+    return p->d_blobs + unit * *bytes;
+}
+
+// a weight pointer of ocb_policy_set_weights_device: 4-byte aligned device (or managed) memory of the handle's device
+static int check_weight_ptr(const ocb_policy* p, int i, const char* name, const float* ptr) {
+    if (ptr == nullptr) return fail(OCB_ERR_INVALID_ARG, "ocb_policy_set_weights_device: src[%d].%s is NULL", i, name);
+    if ((reinterpret_cast<uintptr_t>(ptr) & 3u) != 0)
+        return fail(OCB_ERR_INVALID_ARG, "ocb_policy_set_weights_device: src[%d].%s is not 4-byte aligned", i, name);
+    cudaPointerAttributes at;
+    const cudaError_t err = cudaPointerGetAttributes(&at, ptr);
+    if (err != cudaSuccess) {
+        cudaGetLastError();
+        return fail(OCB_ERR_INVALID_ARG, "ocb_policy_set_weights_device: src[%d].%s: %s", i, name, cudaGetErrorString(err));
+    }
+    if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != p->device)
+        return fail(OCB_ERR_INVALID_ARG, "ocb_policy_set_weights_device: src[%d].%s is not device memory of device %d", i, name,
+                    p->device);
+    return OCB_OK;
+}
+
+// DEVICE fp32 weights -> the same blobs (and zero-observation values) as ocb_policy_set_weights, on `stream`
+extern "C" int ocb_policy_set_weights_device(ocb_policy* p, int n, const ocb_weight_src* src, void* stream) {
+    if (p == nullptr || src == nullptr) return fail(OCB_ERR_INVALID_ARG, "ocb_policy_set_weights_device: NULL argument");
+    if (n < 1) return fail(OCB_ERR_INVALID_ARG, "ocb_policy_set_weights_device: n must be >= 1 (got %d)", n);
+    DeviceGuard guard(p->device);
+    CaptureRelaxed relaxed;  // the pointer queries below while `stream` may be capturing a graph
+    std::vector<uint8_t> seen((size_t)p->n_policies * 2, 0);
+    for (int i = 0; i < n; ++i) {
+        const ocb_weight_src& w = src[i];
+        if (w.policy < 0 || w.policy >= p->n_policies || w.net < 0 || w.net > 1)
+            return fail(OCB_ERR_INVALID_ARG, "ocb_policy_set_weights_device: src[%d] has policy %d / net %d (the handle holds %d sets, "
+                        "nets 0 and 1)", i, w.policy, w.net, p->n_policies);
+        if (seen[(size_t)w.policy * 2 + w.net]++)
+            return fail(OCB_ERR_INVALID_ARG, "ocb_policy_set_weights_device: policy %d net %d appears twice", w.policy, w.net);
+        const char* names[8] = {"conv_w", "conv_b", "fc1_w", "fc1_b", "fc2_w", "fc2_b", "head_w", "head_b"};
+        const float* ptrs[8] = {w.conv_w, w.conv_b, w.fc1_w, w.fc1_b, w.fc2_w, w.fc2_b, w.head_w, w.head_b};
+        for (int k = 0; k < 8; ++k) {
+            const int rc = check_weight_ptr(p, i, names[k], ptrs[k]);
+            if (rc != OCB_OK) return rc;
+        }
+    }
+    PackArgs a;
+    a.fmt = p->generic ? PACK_GENERIC : p->hidden == kH5 ? PACK_H512 : PACK_H64;
+    a.W = p->W, a.H = p->H, a.C = p->C, a.npos = p->npos, a.hidden = p->hidden;
+    a.terrain = p->d_terrain, a.zero_value = p->d_zero_value;
+    blob_of(p, 0, 0, &a.blob_bytes);
+    const size_t units = a.blob_bytes / 16;
+    const unsigned bx = (unsigned)(units < (size_t)kPackThreads * kPackMaxBlocks ? (units + kPackThreads - 1) / kPackThreads
+                                                                                  : kPackMaxBlocks);
+    for (int i0 = 0; i0 < n; i0 += kPackMax) {
+        a.n = n - i0 < kPackMax ? n - i0 : kPackMax;
+        for (int j = 0; j < a.n; ++j) {
+            const ocb_weight_src& w = src[i0 + j];
+            PackDesc& d = a.d[j];
+            size_t bytes;
+            d.dst = blob_of(p, w.policy, w.net, &bytes);
+            d.conv_w = w.conv_w, d.conv_b = w.conv_b, d.fc1_w = w.fc1_w, d.fc1_b = w.fc1_b;
+            d.fc2_w = w.fc2_w, d.fc2_b = w.fc2_b, d.head_w = w.head_w, d.head_b = w.head_b;
+            d.policy = w.policy, d.net = w.net;
+        }
+        policy_pack_kernel<<<dim3(bx + 1, (unsigned)a.n), kPackThreads, 0, (cudaStream_t)stream>>>(a);
+        const cudaError_t err = cudaGetLastError();
+        if (err != cudaSuccess) return fail(OCB_ERR_CUDA, "ocb_policy_set_weights_device: %s", cudaGetErrorString(err));
+    }
+    return OCB_OK;
+}
+
+extern "C" int ocb_policy_read_blob(ocb_policy* p, int policy, int net, void* dst, size_t bytes, void* stream) {
+    if (p == nullptr) return fail(OCB_ERR_INVALID_ARG, "NULL handle");
+    if (policy < 0 || policy >= p->n_policies || net < 0 || net > 1) return fail(OCB_ERR_INVALID_ARG, "bad policy / net index");
+    size_t total;
+    const uint8_t* blob = blob_of(p, policy, net, &total);
+    if (dst == nullptr) return (int)total;
+    if (bytes < total) return fail(OCB_ERR_INVALID_ARG, "ocb_policy_read_blob: dst holds %zu bytes, the blob has %zu", bytes, total);
+    DeviceGuard guard(p->device);
+    const cudaError_t err = cudaMemcpyAsync(dst, blob, total, cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
+    if (err != cudaSuccess) {
+        cudaGetLastError();
+        return fail(OCB_ERR_CUDA, "ocb_policy_read_blob: %s", cudaGetErrorString(err));
+    }
+    return (int)total;
 }
 
 // evaluate_actions extras of ocb_policy_evaluate

@@ -21,7 +21,7 @@ axis order as zero-copy views.
 from __future__ import annotations
 
 import ctypes
-from typing import Dict, Optional
+from typing import Dict, Optional, Sequence
 
 import torch
 
@@ -84,10 +84,15 @@ class MixedPlayCollector:
     ``fused``: ``None`` runs the collection as one persistent launch (``ocb_rollout_mixed_fused``) whenever it applies and
     falls back to the per-step launches for good when the library answers ``OCB_ERR_UNSUPPORTED`` (hidden 512, layouts
     outside the tensor-core kernels or too large for the fused kernel); ``True`` raises ``NativeError`` there instead;
-    ``False`` always runs the per-step path.  ``.fused`` tells which path ran."""
+    ``False`` always runs the per-step path.  ``.fused`` tells which path ran.
+
+    ``weights``: ``(index, actor, critic)`` sets as ``FusedPolicy.set_weights_device`` takes them, refreshed on the device at
+    the start of every ``collect()`` (inside the captured graph with ``use_graph``), as for ``PolicyRollout``.  Slot L of
+    ``value_preds`` is main's critic on the all-zero observation as the handle holds it when the collection runs."""
 
     def __init__(self, env: B200Overcooked, policy: FusedPolicy, L: int, main_policy: int = 0, partner_policy: int = 1,
-                 seed: int = 0, mix_seed: int = 0, use_graph: bool = False, fused: Optional[bool] = None):
+                 seed: int = 0, mix_seed: int = 0, use_graph: bool = False, fused: Optional[bool] = None,
+                 weights: Optional[Sequence] = None):
         if env.num_players != 2:
             raise ValueError("mixed play supports 2 players")
         if env.sim_device != policy.device:
@@ -99,6 +104,10 @@ class MixedPlayCollector:
                              "exactly L - 1)" % (L - 1))
         if not (0 <= main_policy < policy.n_policies and 0 <= partner_policy < policy.n_policies):
             raise ValueError("policy index out of range")
+        self.weights = None
+        if weights is not None:
+            self.weights = list(weights)
+            policy._weight_srcs(self.weights)  # shape / dtype / device errors now rather than at the first collect
         self.env, self.policy, self.L = env, policy, L
         self.main_policy, self.partner_policy = main_policy, partner_policy
         self.seed, self.mix_seed = seed, mix_seed
@@ -121,6 +130,8 @@ class MixedPlayCollector:
         stream = ctypes.c_void_p(torch.cuda.current_stream(env.sim_device).cuda_stream)
         # launch-local sampling rows (a sharded PolicyRollout may have left global rows on a shared policy handle)
         _native.check(self._lib.ocb_policy_set_sampling_rows(self.policy._h, 0, 0, 0))
+        if self.weights is not None:
+            self.policy.set_weights_device(self.weights)
         if self.fused:
             rc = self._lib.ocb_rollout_mixed_fused(
                 env._h, self.policy._h, self.L, self.main_policy, self.partner_policy, _ptr(b.obs), _ptr(b.actions),

@@ -21,6 +21,7 @@ import torch.nn.functional as F
 
 NUM_ACTIONS = 6
 _BASE_KEYS = ("base.cnn.cnn.0", "base.cnn.cnn.3", "base.cnn.cnn.5")
+_WEIGHTS = ("conv_w", "conv_b", "fc1_w", "fc1_b", "fc2_w", "fc2_b", "head_w", "head_b")  # in state_dict() order
 
 
 class PolicyNet:
@@ -83,6 +84,36 @@ class PolicyNet:
             if tuple(src.shape) != tuple(dst.shape):
                 raise ValueError("%s: shape %s, expected %s" % (k, tuple(src.shape), tuple(dst.shape)))
             dst.copy_(src)
+        return self
+
+    def alias_state_dict(self, sd) -> "PolicyNet":
+        """Like ``load_state_dict``, but the net keeps references to the given tensors instead of copying them.  A net
+        built from ``module.state_dict()`` of the reference's ``R_Actor`` / ``R_Critic`` therefore sees the optimizer's
+        in-place updates, and ``FusedPolicy.set_weights_device`` (or a collector given ``weights=``) packs the current
+        values.  Each tensor must have its shape, be fp32 and contiguous, and live on this net's device (``ValueError``)."""
+        mine = self.state_dict()
+        missing = [k for k in mine if k not in sd]
+        if missing:
+            raise KeyError("state dict lacks %s" % missing)
+        want = self.device
+        if want.type == "cuda" and want.index is None:
+            want = torch.device("cuda", torch.cuda.current_device())
+        keep = []
+        for k, dst in mine.items():
+            src = sd[k]
+            if not isinstance(src, torch.Tensor):
+                raise ValueError("%s: expected a tensor, got %s" % (k, type(src).__name__))
+            if tuple(src.shape) != tuple(dst.shape):
+                raise ValueError("%s: shape %s, expected %s" % (k, tuple(src.shape), tuple(dst.shape)))
+            if src.dtype != torch.float32:
+                raise ValueError("%s: dtype %s, expected torch.float32" % (k, src.dtype))
+            if not src.is_contiguous():
+                raise ValueError("%s is not contiguous" % k)
+            if src.device != want:
+                raise ValueError("%s lives on %s, this net on %s" % (k, src.device, want))
+            keep.append(src.detach())
+        for name, t in zip(_WEIGHTS, keep):
+            setattr(self, name, t)
         return self
 
     # ------------------------------------------------------------------ fp32 reference forward
@@ -148,6 +179,57 @@ class FusedPolicy:
                   (net.conv_w, net.conv_b, net.fc1_w, net.fc1_b, net.fc2_w, net.fc2_b, net.head_w, net.head_b)]
             ptrs = [self._ct.c_void_p(t.data_ptr()) for t in ts]
             self._native.check(self._lib.ocb_policy_set_weights(self._h, index, net_id, *ptrs))
+
+    def _weight_srcs(self, sets):
+        """``ocb_weight_src`` array of ``set_weights_device``; checks every tensor against this handle's shapes"""
+        h, co = self.hidden, self.hidden // 2
+        npos = (self.layout.width - 2) * (self.layout.height - 2)
+        descs = []
+        for index, actor, critic in sets:
+            if not 0 <= int(index) < self.n_policies:
+                raise ValueError("weight set %d out of range (the handle holds %d)" % (int(index), self.n_policies))
+            for net_id, net in ((0, actor), (1, critic)):
+                if net is None:
+                    continue
+                out = NUM_ACTIONS if net_id == 0 else 1
+                shapes = ((co, self.layout.channels, 3, 3), (co,), (h, co * npos), (h,), (h, h), (h,), (out, h), (out,))
+                ts = [getattr(net, name) for name in _WEIGHTS]
+                for name, t, shape in zip(_WEIGHTS, ts, shapes):
+                    if tuple(t.shape) != shape:
+                        raise ValueError("%s of set %d net %d: shape %s, expected %s" % (name, index, net_id, tuple(t.shape), shape))
+                    if t.dtype != torch.float32:
+                        raise ValueError("%s of set %d net %d: dtype %s, expected torch.float32" % (name, index, net_id, t.dtype))
+                    if not t.is_contiguous():
+                        raise ValueError("%s of set %d net %d is not contiguous" % (name, index, net_id))
+                    if t.device != self.device:
+                        raise ValueError("%s of set %d net %d lives on %s, the handle on %s" % (name, index, net_id, t.device,
+                                                                                           self.device))
+                descs.append((int(index), net_id, ts))
+        if not descs:
+            raise ValueError("no network to refresh")
+        arr = (self._native.ocb_weight_src * len(descs))()
+        for d, (index, net_id, ts) in zip(arr, descs):
+            d.policy, d.net = index, net_id
+            for name, t in zip(_WEIGHTS, ts):
+                setattr(d, name, t.data_ptr())
+        return arr
+
+    def set_weights_device(self, sets):
+        """``set_weights`` for weights already on this handle's device: ``sets`` is a sequence of ``(index, actor, critic)``
+        (either net may be ``None``), packed into the same bytes ``set_weights`` writes, in ONE native call on torch's
+        current stream (``ocb_policy_set_weights_device``).  Nothing synchronises, so the refresh is ordered with the
+        collections around it and can be captured into a CUDA graph; the weights are read when it runs."""
+        arr = self._weight_srcs(sets)
+        with torch.cuda.device(self.device):
+            self._native.check(self._lib.ocb_policy_set_weights_device(self._h, len(arr), arr, self._stream()))
+
+    def read_blob(self, index: int, net: int) -> torch.Tensor:
+        """the packed bytes of (weight set, net) as a uint8 device tensor (``ocb_policy_read_blob``, diagnostic)"""
+        n = self._native.check(self._lib.ocb_policy_read_blob(self._h, index, net, None, 0, None))
+        out = torch.empty((n,), dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            self._native.check(self._lib.ocb_policy_read_blob(self._h, index, net, self._p(out), n, self._stream()))
+        return out
 
     def _p(self, t):
         return None if t is None else self._ct.c_void_p(t.data_ptr())

@@ -131,7 +131,8 @@ class PolicyRollout:
     def __init__(self, env: B200Overcooked, policy: FusedPolicy, T: int, tile_policy: Optional[torch.Tensor] = None,
                  with_critic: bool = True, with_logp: bool = True, seed: int = 0, use_graph: bool = False,
                  fused: Optional[bool] = None, policy_index: int = 0, world_offset: int = 0,
-                 total_worlds: Optional[int] = None, critic_policy: Optional[torch.Tensor] = None):
+                 total_worlds: Optional[int] = None, critic_policy: Optional[torch.Tensor] = None,
+                 weights: Optional[Sequence] = None):
         """``total_worlds`` (with ``world_offset`` = global index of this env's world 0): key the action sampling by
         the GLOBAL (seat, world) so that a sharded run draws exactly the streams of the unsharded one
         (``ocb_policy_set_sampling_rows``); ``None`` keeps the launch-local rows.
@@ -151,7 +152,12 @@ class PolicyRollout:
         (``ocb_rollout_crossplay_train_fused``), falling back to per-step actor launches and per-step critic passes where
         that is unsupported (hidden 512, layouts outside the fused kernel); ``fused=True`` raises ``NativeError`` there.
         Both tables are checked once, here (entries -1 or below ``n_policies``; ``tile_policy`` entries 0 or more); the
-        launches read the caller's tensors."""
+        launches read the caller's tensors.
+
+        ``weights``: ``(index, actor, critic)`` sets as ``FusedPolicy.set_weights_device`` takes them.  Every ``collect()``
+        then first packs their current values into the handle on the device, in the same stream as the collection; with
+        ``use_graph`` the refresh is part of the captured graph, so one replay loads the parameters the nets hold at that
+        moment (nets made with ``PolicyNet.alias_state_dict`` follow the trainer's optimizer) and collects with them."""
         if env.num_players != policy.layout.num_players:
             raise ValueError("env and policy were built for different player counts")
         if env.sim_device != policy.device:
@@ -175,6 +181,10 @@ class PolicyRollout:
                 host = table.cpu()
                 if bool(((host < low) | (host >= policy.n_policies)).any()):
                     raise ValueError("%s entries must lie in [%d, %d)" % (name, low, policy.n_policies))
+        self.weights = None
+        if weights is not None:
+            self.weights = list(weights)
+            policy._weight_srcs(self.weights)  # shape / dtype / device errors now rather than at the first collect
         self.env, self.policy, self.T, self.seed = env, policy, T, seed
         self.tile_policy, self.critic_policy = tile_policy, critic_policy
         self.buf = RolloutBuffer(env, T, with_critic, with_logp)
@@ -230,6 +240,8 @@ class PolicyRollout:
         stream = ctypes.c_void_p(torch.cuda.current_stream(env.sim_device).cuda_stream)
         # handle-level state, set per issue: several rollouts may share one policy handle
         _native.check(self._lib.ocb_policy_set_sampling_rows(self.policy._h, *self._sampling_rows))
+        if self.weights is not None:
+            self.policy.set_weights_device(self.weights)
         if self.fused:
             if self.critic_policy is not None:
                 rc = self._lib.ocb_rollout_crossplay_train_fused(

@@ -204,6 +204,24 @@ int ocb_policy_destroy(ocb_policy* pol);
 int ocb_policy_set_weights(ocb_policy* pol, int policy, int net, const float* conv_w, const float* conv_b,
                            const float* fc1_w, const float* fc1_b, const float* fc2_w, const float* fc2_b,
                            const float* head_w, const float* head_b);
+/* One network for ocb_policy_set_weights_device: weight set `policy`, net 0 (actor) or 1 (critic), and DEVICE fp32 tensors in
+ * the layouts ocb_policy_set_weights takes (contiguous, 4-byte aligned, on the handle's device). */
+typedef struct ocb_weight_src {
+    int policy, net;
+    const float *conv_w, *conv_b, *fc1_w, *fc1_b, *fc2_w, *fc2_b, *head_w, *head_b;
+} ocb_weight_src;
+/* ocb_policy_set_weights for n networks whose weights are already on the device (e.g. a trainer's parameters after an
+ * optimizer step): packs them into the handle's blobs, byte for byte what ocb_policy_set_weights writes for the same values
+ * (the critic's zero-observation value included), in one launch on `stream` (more than a launch's parameter block holds are
+ * split over a few).  `src` is a HOST array of n descriptors, read during the call; the weights are read when the launch
+ * runs.  Nothing synchronises and nothing is allocated, so the call can be captured into a CUDA graph, whose replays then
+ * pack whatever the tensors hold at replay time.  Every argument is checked before anything is launched: NULL handle or
+ * array, n < 1, a policy / net out of range, the same (policy, net) twice, and a NULL, unaligned or non-device pointer
+ * are OCB_ERR_INVALID_ARG.  Extents cannot be checked here: each tensor must hold its layout's element count. */
+int ocb_policy_set_weights_device(ocb_policy* pol, int n, const ocb_weight_src* src, void* stream);
+/* diagnostic: copies the packed blob of (policy, net) to dst (DEVICE, at least the blob's size) on `stream` and returns its
+ * size in bytes; dst NULL only returns the size */
+int ocb_policy_read_blob(ocb_policy* pol, int policy, int net, void* dst, size_t bytes, void* stream);
 /* actor: obs int8 [M, W, H, C] (DEVICE) -> sampled (or arg-max) actions int32 [M], log-probs
  * float [M], raw logits float [M,6]; any output may be NULL.  tile_policy int32 [ceil(M/128)]
  * selects the weight set per 128-row tile (NULL = set 0) — the cross-play slice multiplexing of
